@@ -1,8 +1,13 @@
 #!/usr/bin/env python
 """bench.py -- motion-module throughput of one UNet denoising step (BASELINE.json config 2) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes the 20 module outputs of the last timed step (rank 0) as DIR/<call>.npy, float32: a fixed sample of
+DUMP_ELEMS elements of each output's logical [B,C,F,H,W] order, the positions seeded by the output's size. The inputs come from a
+generator of their own and the weights from name-keyed seeds (oracle.motion_oracle.make_params), so they do not depend on how a
+build constructs its modules: two builds run with the same arguments can be compared output for output.
 
 A "step" = the 20 motion-module calls of one UNet3DConditionModel.forward at SD1.5 512x512 (64x64 latent), 8 frames,
 CFG batch 2, bf16 -- 20 distinct modules (417 M parameters), 20 distinct [2,C,8,L,L] activations in the
@@ -36,6 +41,7 @@ sys.path.insert(0, ROOT)
 
 LATENT, FRAMES, BATCH = 64, 8, 2
 METRIC, UNIT = "motion-module fwd TFLOP/s", "TFLOP/s"
+DUMP_ELEMS = 1 << 19          # per output: 20 x 2 MiB of float32, under 64 MB in all
 
 
 def workload_config(n_gpus):
@@ -108,6 +114,17 @@ def measured_peaks():
         return {"bf16_tflops": p.get("bf16_tflops"), "bf16_tflops_sustained": p.get("bf16_tflops_sustained"),
                 "hbm_gbs": p.get("hbm_gbs"), "source": "measured (MEASURED_PEAKS.json)"}
     return {"bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "hbm_gbs": 6650.0, "source": "fallback (B200_PROFILING.md)"}
+
+
+def dump_positions(calls):
+    """{output size: DUMP_ELEMS sorted positions in the logical [B,C,F,H,W] order}, seeded by the size alone, so that the sample is
+    the same in every run and every build."""
+    positions = {}
+    for c in calls:
+        n = BATCH * c.channels * FRAMES * c.side * c.side
+        if n not in positions:
+            positions[n] = torch.randperm(n, generator=torch.Generator().manual_seed(n))[:DUMP_ELEMS].sort().values
+    return positions
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -431,7 +448,12 @@ def main():
     ap.add_argument("--no-clips", action="store_true", help="skip the 25-step clip loop (secondary metric)")
     ap.add_argument("--no-eager", action="store_true", help="skip the stock-torch-eager GPU anchor")
     ap.add_argument("--no-spatial", action="store_true", help="skip the spatial-transformer leg (SURVEY 8(f) N3, secondary metric)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last timed step's outputs to DIR/<call>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours only")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -460,14 +482,18 @@ def main():
     kwargs = dict(num_attention_heads=8, num_transformer_block=1, attention_block_types=("Temporal_Self", "Temporal_Self"),
                   temporal_position_encoding=True, temporal_position_encoding_max_len=24, temporal_attention_dim_div=1,
                   zero_initialize=False)      # random-init weights of the v3 architecture; proj_out NOT zeroed (else identity)
-    torch.manual_seed(1234 + rank)
+    from oracle import motion_oracle as mo          # seeded weights only; never the product path
+    seed = 1234 + rank
+    torch.manual_seed(seed)
+    gen = torch.Generator(device=dev).manual_seed(seed)
     modules, xs_dev, xs_host, ys_host = [], [], [], []
     with torch.no_grad():
-        for c in calls:
+        for i, c in enumerate(calls):
             with torch.device(dev):
                 m = nb.get_motion_module(c.channels, "Vanilla", kwargs)
+            m.load_state_dict(mo.make_params(mo.MotionConfig(c.channels, 8, 1, c.attn_blocks, True, c.max_len), seed * 64 + i))
             modules.append(m.to(torch.bfloat16).eval())
-            x = torch.randn(BATCH, FRAMES, c.channels, c.side, c.side, device=dev, dtype=torch.bfloat16).permute(0, 2, 1, 3, 4)
+            x = torch.randn(BATCH, FRAMES, c.channels, c.side, c.side, device=dev, dtype=torch.bfloat16, generator=gen).permute(0, 2, 1, 3, 4)
             xs_dev.append(x)
             xs_host.append(torch.empty((BATCH, FRAMES, c.channels, c.side, c.side), dtype=torch.bfloat16).pin_memory())
             xs_host[-1].copy_(x.permute(0, 2, 1, 3, 4))
@@ -475,9 +501,15 @@ def main():
     h2d_bytes = sum(t.numel() * 2 for t in xs_host)
     d2h_bytes = sum(t.numel() * 2 for t in ys_host)
 
-    def step_resident():
+    def step_resident(keep=False):
+        # an output is dropped as soon as the next call is issued (its buffer then takes the next output, as in a UNet that consumes
+        # it right away); keep=True returns them instead
+        ys = []
         for m, x in zip(modules, xs_dev):
-            m(x, None, None)
+            y = m(x, None, None)
+            if keep:
+                ys.append(y)
+        return ys
 
     def barrier():
         torch.cuda.synchronize()
@@ -487,20 +519,26 @@ def main():
 
     with torch.no_grad():
         # ---------------- device-resident arm ("value") ----------------
-        for _ in range(args.warmup):
-            step_resident()
+        # --dump-outputs: the last step of each loop keeps its outputs, the warm-up's so that the allocator already holds 20 output
+        # buffers when the timed region reaches its own last step, the one that is written
+        positions = {n: p.to(dev) for n, p in dump_positions(calls).items()} if args.dump_outputs else None
+        for i in range(args.warmup):
+            step_resident(keep=positions is not None and i == args.warmup - 1)
         barrier()
         sampler = ClockSampler(physical_gpu_index(local_rank))
         sampler.start()
         launches0 = nb.launch_count()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
-        for _ in range(args.steps):
-            step_resident()
+        for i in range(args.steps):
+            ys = step_resident(keep=positions is not None and i == args.steps - 1)
         ev1.record()
         barrier()
         ms_total = ev0.elapsed_time(ev1)
         launches = nb.launch_count() - launches0
+        # sampled on the device at once, so that the outputs do not outlive the timed region
+        dumped = [y.reshape(-1).index_select(0, positions[y.numel()]).float().cpu().numpy() for y in ys] if positions else None
+        del ys
         # ---------------- same K steps again with the library's per-kernel CUDA events (roofline of the dominant kernel) --------
         # (kept out of the `value` region: an event between two kernels defeats programmatic dependent launch)
         nlib.profile_begin()
@@ -665,6 +703,11 @@ def main():
                     if eager and "bf16" in eager and "ms_per_step" in spatial.get("gpu_eager_baseline", {}) else None},
                 "flops_per_step": flops_step}
         print(json.dumps(line), flush=True)
+        if dumped is not None:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for i, (c, a) in enumerate(zip(calls, dumped)):
+                np.save(os.path.join(args.dump_outputs, f"call{i:02d}_c{c.channels}_{c.side}x{c.side}.npy"), a)
     if world > 1:
         dist.destroy_process_group()
 
