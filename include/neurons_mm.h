@@ -310,7 +310,9 @@ NMM_API int nmm_spatial_forward_stats(const nmm_spatial_shape *s, const void *x,
  * motion_module_new.py:258-287, with the head split / merge of :181-193 folded into the indexing.  q: `images` x [q_len rows] of
  * heads * head_dim channels at the given row / image strides (elements); k, v: [kv_len rows] per kv image, kv image of q image i =
  * i / kv_div (kv_div = frames for the text cross-attention, 1 for self-attention); o like q.  dtype NMM_BF16 (tensor cores; 16-byte
- * aligned, strides % 8 == 0) or NMM_F32 (fp32 checker kernel).  head_dim in {40, 80, 160}. */
+ * aligned, strides % 8 == 0), NMM_F32 (fp32 checker kernel) or NMM_F32X3 (fp32-grade, 3 bf16 MMAs per product): q, k, v are then
+ * bf16 rows of a hi plane and a lo plane, the lo plane half a row stride after the hi plane (e.g. q rows [hi q | lo q], k | v rows
+ * [hi k | hi v | lo k | lo v]), o is fp32.  head_dim in {40, 80, 160}. */
 NMM_API int nmm_spatial_attention(int32_t dtype, const void *q, const void *k, const void *v, void *o, int64_t q_row_stride, int64_t kv_row_stride,
                                   int64_t o_row_stride, int64_t q_image_stride, int64_t kv_image_stride, int64_t o_image_stride, int32_t q_len,
                                   int32_t kv_len, int32_t heads, int32_t head_dim, int32_t images, int32_t kv_div, void *stream);

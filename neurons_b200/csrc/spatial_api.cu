@@ -190,6 +190,11 @@ int nmm_spatial_attention(int32_t dtype, const void *q, const void *k, const voi
     a.Lq = q_len; a.Lkv = kv_len; a.heads = heads; a.images = images; a.kv_div = kv_div; a.dh = head_dim; a.dtype = dtype;
     a.scale = 1.0f / sqrtf((float)head_dim);
     a.scale_log2e = a.scale * 1.4426950408889634f;
+    if (dtype == NMM_F32X3) {      // q, k, v: bf16 hi | lo planes, the lo plane half a row stride after the hi plane (spatial_forward_impl's layout); o: fp32
+        if (q_row_stride % 2 || kv_row_stride % 2) return fail(NMM_ERR_BAD_ARG, "NMM_F32X3 spatial attention: row strides must be even (hi | lo planes)");
+        a.q_lo_off = q_row_stride / 2; a.kv_lo_off = kv_row_stride / 2;
+        return launch_spatial_attention_x3(a, (cudaStream_t)stream);
+    }
     return launch_spatial_attention(a, (cudaStream_t)stream);
 }
 

@@ -242,9 +242,11 @@ def spatial_forward_packed(x: torch.Tensor, encoder_hidden_states: torch.Tensor,
     return out
 
 
-def spatial_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int, kv_div: int = 1) -> torch.Tensor:
+def spatial_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int, kv_div: int = 1, x3: bool = False) -> torch.Tensor:
     """Per-stage entry (tests / micro-benchmarks): q [images, Lq, heads*dh], k / v [images / kv_div, Lkv, heads*dh] (last dim dense; row
-    and image strides free) -> o [images, Lq, heads*dh].  nmm_spatial_attention."""
+    and image strides free) -> o [images, Lq, heads*dh].  nmm_spatial_attention.
+    x3=True (fp32 q, k, v): the fp32-grade tensor-core kernel of the NMM_F32X3 mode -- q and k | v are converted to hi | lo planes here
+    (like ops.linear(..., x3=True)); o is fp32."""
     for t, name in ((q, "q"), (k, "k"), (v, "v")):
         ops._require_cuda(t, name)
         if t.dim() != 3 or t.stride(2) != 1:
@@ -252,9 +254,17 @@ def spatial_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: 
     images, Lq, Cc = q.shape
     if k.shape != v.shape or k.stride() != v.stride() or k.shape[0] * kv_div != images or k.shape[2] != Cc:
         raise ValueError("k / v must share shape and strides, with images == kv images * kv_div")
-    o = torch.empty((images, Lq, Cc), dtype=q.dtype, device=q.device)
+    dt = _dtype_code(q.dtype)
+    if x3:
+        if q.dtype != torch.float32 or k.dtype != torch.float32 or v.dtype != torch.float32:
+            raise TypeError("spatial_attention(x3=True) takes fp32 q, k, v")
+        Lkv = k.shape[1]
+        q = ops.split_planes(q.reshape(images * Lq, Cc)).view(images, Lq, 2 * Cc)                      # rows [hi q | lo q]
+        kv = ops.split_planes(torch.cat([k, v], -1).reshape(-1, 2 * Cc)).view(-1, Lkv, 4 * Cc)        # rows [hi k | hi v | lo k | lo v]
+        k, v, dt = kv[..., :Cc], kv[..., Cc:2 * Cc], _lib.NMM_F32X3
+    o = torch.empty((images, Lq, Cc), dtype=torch.float32 if x3 else q.dtype, device=q.device)
     with torch.cuda.device(q.device):
-        _lib.check(_lib.load().nmm_spatial_attention(_dtype_code(q.dtype), q.data_ptr(), k.data_ptr(), v.data_ptr(), o.data_ptr(), q.stride(1), k.stride(1),
+        _lib.check(_lib.load().nmm_spatial_attention(dt, q.data_ptr(), k.data_ptr(), v.data_ptr(), o.data_ptr(), q.stride(1), k.stride(1),
                                                      o.stride(1), q.stride(0), k.stride(0), o.stride(0), Lq, k.shape[1], heads, Cc // heads, images,
                                                      kv_div, ops._stream_ptr(q.device)))
     return o
