@@ -128,7 +128,8 @@ typedef enum nmm_option {
                                    a statistics pass over the (L2-resident) y, measured faster there.  env NMM_FUSED_Y_STATS          */
     NMM_OPT_FUSED_CLUSTER = 9,  /* 0: CTA pairs when the tile count is even; 1: force the single-CTA fused kernel.  env NMM_FUSED_CLUSTER */
     NMM_OPT_SPATIAL_ATTN = 10,  /* spatial self-attention (d_h 40 / 80, >= 256 keys): 0 = tcgen05 kernel (planner: two query tiles per CTA); 1 = mma.sync kernel;
-                                   other values: A/B variants of the tcgen05 kernel (csrc/spatial_attention_tc.cu).  env NMM_SPATIAL_ATTN */
+                                   other values: A/B variants of the tcgen05 kernel (csrc/spatial_attention_tc.cu).  fp32 calls (NMM_F32): 30 = always the
+                                   tiled FMA-pipe kernel, 31 = always the one-warp-per-query checker; other values select by size.  env NMM_SPATIAL_ATTN */
     NMM_OPT_COUNT = 11
 } nmm_option;
 NMM_API int nmm_set_option(int32_t option, int64_t value);

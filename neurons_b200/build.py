@@ -20,7 +20,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libneurons_mm.so")
-SOURCES = ["api.cu", "norm_kernels.cu", "attention_kernel.cu", "gemm_simt.cu", "gemm_tcgen05.cu", "sampler_kernels.cu", "fused_module.cu", "spatial_attention.cu", "spatial_attention_tc.cu", "spatial_attention_x3.cu", "spatial_api.cu", "decoder_attention.cu"]
+SOURCES = ["api.cu", "norm_kernels.cu", "attention_kernel.cu", "gemm_simt.cu", "gemm_tcgen05.cu", "sampler_kernels.cu", "fused_module.cu", "spatial_attention.cu", "spatial_attention_tc.cu", "spatial_attention_x3.cu", "spatial_attention_f32.cu", "spatial_api.cu", "decoder_attention.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

@@ -265,13 +265,15 @@ struct FlashArgs {
     int64_t q_bs, kv_bs, o_bs;      // image strides (elements); the k / v image of q image i is i / kv_div
     int64_t q_lo_off, kv_lo_off;    // launch_spatial_attention_x3 only: element offset of the lo plane inside a q / k-v row (hi | lo planes)
     int Lq, Lkv, heads, images, kv_div, dh;
-    int dtype;                      // NMM_BF16 (mma.sync flash kernel) or NMM_F32 (fp32 checker kernel)
+    int dtype;                      // NMM_BF16 (mma.sync flash kernel) or NMM_F32 (fp32 kernels: tiled FMA-pipe flash or checker)
     float scale, scale_log2e;       // dh^-1/2 and dh^-1/2 * log2(e)
 };
 int launch_spatial_attention(const FlashArgs &a, cudaStream_t st);
 bool spatial_attention_tc_eligible(const FlashArgs &a);                            // spatial_attention_tc.cu (tcgen05 / TMEM / TMA)
 int launch_spatial_attention_tc(const FlashArgs &a, int variant, cudaStream_t st);
 int launch_spatial_attention_x3(const FlashArgs &a, cudaStream_t st);               // spatial_attention_x3.cu: fp32-grade (hi | lo bf16 planes in, fp32 out)
+bool spatial_attention_f32_tiled_eligible(const FlashArgs &a);                      // spatial_attention_f32.cu: NMM_F32 flash kernel on the FMA pipe
+int launch_spatial_attention_f32_tiled(const FlashArgs &a, cudaStream_t st);
 int device_check();
 
 // GEMM + epilogue

@@ -232,8 +232,9 @@ __global__ void __launch_bounds__(32 * WARPS, DH <= 80 ? 16 / WARPS : 8 / WARPS)
     }
 }
 
-// fp32 checker path (NMM_F32): one warp per (query, head); lanes split the keys, fp32 throughout.  Slow by design -- it exists so
-// that the fp32 parity mode of the spatial transformer has no bf16 rounding anywhere (bar 1e-4), like the FMA-pipe GEMM.
+// fp32 checker path (NMM_F32, small shapes): one warp per (query, head); lanes split the keys, fp32 throughout -- so that the fp32 parity
+// mode of the spatial transformer has no bf16 rounding anywhere (bar 1e-4), like the FMA-pipe GEMM.  Large shapes run the tiled kernel of
+// spatial_attention_f32.cu, which keeps this arithmetic.
 template <int DH>
 __global__ void __launch_bounds__(128) spatial_attention_f32_kernel(const float *__restrict__ q, const float *__restrict__ k, const float *__restrict__ v,
                                                                      float *__restrict__ o, int64_t q_rs, int64_t kv_rs, int64_t o_rs, int64_t q_bs,
@@ -326,11 +327,20 @@ int launch_spatial_attention(const FlashArgs &a, cudaStream_t st) {
             default: break;
         }
     } else if (a.dtype == NMM_F32) {
-        // the fp32 kernel is the CHECKER (one warp per query, keys streamed from L2): fine at test sizes, minutes at the 64 x 64 level.
-        // Refuse instead of appearing to hang; bf16 is the production mode of the spatial transformer.
-        if ((double)a.Lq * a.Lkv * a.images * a.heads > 1.1e9)
-            return fail(NMM_ERR_UNSUPPORTED, "fp32 spatial attention is a checker for small shapes (%d x %d keys x %d images x %d heads is too large): "
-                        "run the spatial transformer in bf16", a.Lq, a.Lkv, a.images, a.heads);
+        // Two kernels with the same arithmetic: the tiled flash kernel on the FMA pipe (spatial_attention_f32.cu) from F32_TILED_MIN_SCORES
+        // score elements up, the checker (one warp per query, keys streamed from L2) below.  Measured on B200 the tiled kernel is the faster
+        // one at every swept size, from 8e3 score elements up (1.5-4x at 1e4-1e5, 45-65x from 1e7; profiles/r3_spatial_fp32_attention.txt).
+        // The checker is kept below 2^17, where a call costs 0.02-0.26 ms either way, so that small fp32 calls (the parity fixtures, the
+        // tests) keep the results of earlier releases bit for bit.
+        constexpr double F32_TILED_MIN_SCORES = 1 << 17;
+        const double scores = (double)a.Lq * a.Lkv * a.images * a.heads;
+        const bool tiled = spatial_attention_f32_tiled_eligible(a);
+        if (variant == 30 && !tiled) return fail(NMM_ERR_BAD_ARG, "fp32 tiled spatial attention needs 16-byte aligned q / k / v with strides in multiples of 4");
+        if (tiled && variant != 31 && (variant == 30 || scores >= F32_TILED_MIN_SCORES)) return launch_spatial_attention_f32_tiled(a, st);
+        // the checker takes minutes at the 64 x 64 level: refuse misaligned operands there instead of appearing to hang
+        if (variant != 31 && scores > 1.1e9)
+            return fail(NMM_ERR_UNSUPPORTED, "fp32 spatial attention of %d x %d keys x %d images x %d heads needs 16-byte aligned q / k / v with "
+                        "strides in multiples of 4 (the tiled kernel)", a.Lq, a.Lkv, a.images, a.heads);
         switch (a.dh) {
             case 40: return launch_flash_f32_t<40>(a, st);
             case 80: return launch_flash_f32_t<80>(a, st);

@@ -38,8 +38,8 @@ class SpatialConfig:
     layers: int = 1
     ctx_dim: int = 768
     # fp32 activations: True = every Linear on the tensor cores as 3 bf16 MMAs per product (NMM_F32X3; needs channels, ctx_dim % 64 == 0),
-    # False (module flag `_nmm_fp32_fma` or env NMM_FP32_FMA=1) = the FMA-pipe GEMM (NMM_F32), the checker.  The attention itself is the
-    # fp32 checker kernel in both modes (small / medium shapes; the 64 x 64 level is refused in fp32: use bf16 there).
+    # False (module flag `_nmm_fp32_fma` or env NMM_FP32_FMA=1) = the FMA-pipe GEMM (NMM_F32) and fp32 attention on the FMA pipe (no bf16
+    # rounding anywhere; the tiled flash kernel at every UNet size, the one-warp-per-query checker kernel for small shapes).
     fp32_tc: bool = True
 
 
@@ -245,6 +245,8 @@ def spatial_forward_packed(x: torch.Tensor, encoder_hidden_states: torch.Tensor,
 def spatial_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int, kv_div: int = 1, x3: bool = False) -> torch.Tensor:
     """Per-stage entry (tests / micro-benchmarks): q [images, Lq, heads*dh], k / v [images / kv_div, Lkv, heads*dh] (last dim dense; row
     and image strides free) -> o [images, Lq, heads*dh].  nmm_spatial_attention.
+    fp32 q, k, v (x3=False): fp32 throughout on the FMA pipe, the attention of the FMA mode -- the tiled flash kernel from 2^17 score elements
+    (Lq * Lkv * images * heads) up, the checker kernel below; q, k, v need 16-byte alignment and strides in multiples of 4 for the tiled kernel.
     x3=True (fp32 q, k, v): the fp32-grade tensor-core kernel of the NMM_F32X3 mode -- q and k | v are converted to hi | lo planes here
     (like ops.linear(..., x3=True)); o is fp32."""
     for t, name in ((q, "q"), (k, "k"), (v, "v")):

@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Max-abs error of the attention kernels against fp64 as the logits grow: the spatial kernels (bf16 tcgen05, fp32-grade x3, fp32 checker)
+"""Max-abs error of the attention kernels against fp64 as the logits grow: the spatial kernels (bf16 tcgen05, fp32-grade x3, fp32 checker, fp32 tiled)
 and the temporal attention (bf16, fp32), on randn q scaled to a given max |logit| (tests/test_attention_edges.py `peaked`), |v| ~ N(0, 1).
 For x3 it also prints what an fp64 emulation of the kernel's own arithmetic predicts (split, 3 products, fp32 scores, split weights), and for
 reference what fp32 torch on the host gives.  Prints the GPU's name and power limit first.  Development / profiles tool."""
@@ -12,6 +12,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import neurons_b200 as nb  # noqa: E402
+from neurons_b200 import lib as nlib  # noqa: E402
 from neurons_b200 import ops  # noqa: E402
 from oracle import motion_oracle as mo  # noqa: E402
 from tests import test_attention_edges as te  # noqa: E402
@@ -38,7 +39,7 @@ def main():
         pl = "unknown"
     print(f"# {name}, power limit {pl}")
     print("# spatial: 2 images x 2 heads, Lq 256, Lkv 1024 (x3 / fp32: Lq 128), q = randn scaled to max |logit|, k, v = randn")
-    print(f"{'dh':>4} {'max|logit|':>10} {'bf16 tc':>10} {'x3':>10} {'x3 emul.':>10} {'fp32 chk':>10} {'torch fp32':>10}")
+    print(f"{'dh':>4} {'max|logit|':>10} {'bf16 tc':>10} {'x3':>10} {'x3 emul.':>10} {'fp32 chk':>10} {'fp32 tiled':>10} {'torch fp32':>10}")
     for dh in (40, 80, 160):
         for L in LOGITS:
             q, k, v = te.make_case("peaked", 256, 1024, 2, dh, seed=dh + L, logit=float(L))
@@ -49,9 +50,12 @@ def main():
             ref = te.attention_fp64(q, k, v, 2)
             e_x3 = err(nb.spatial_attention(q.cuda(), k.cuda(), v.cuda(), 2, x3=True), ref)
             e_emu = err(te.x3_emulation(q, k, v, 2), ref)
-            e_f32 = err(nb.spatial_attention(q.cuda(), k.cuda(), v.cuda(), 2), ref)
+            with nlib.options({nlib.OPT_SPATIAL_ATTN: 31}):          # NMM_F32: force the checker / the tiled kernel
+                e_f32 = err(nb.spatial_attention(q.cuda(), k.cuda(), v.cuda(), 2), ref)
+            with nlib.options({nlib.OPT_SPATIAL_ATTN: 30}):
+                e_tiled = err(nb.spatial_attention(q.cuda(), k.cuda(), v.cuda(), 2), ref)
             e_t = err(torch_fp32(q, k, v, 2, 1), ref)
-            print(f"{dh:>4} {L:>10} {e_bf16:>10.2e} {e_x3:>10.2e} {e_emu:>10.2e} {e_f32:>10.2e} {e_t:>10.2e}", flush=True)
+            print(f"{dh:>4} {L:>10} {e_bf16:>10.2e} {e_x3:>10.2e} {e_emu:>10.2e} {e_f32:>10.2e} {e_tiled:>10.2e} {e_t:>10.2e}", flush=True)
     print("# temporal: B 1, 3 x 3 positions, 8 heads; qkv randn with q scaled to max |logit|; kernel of NMM_OPT_ATTN_VARIANT 0")
     print(f"{'C':>5} {'F':>3} {'max|logit|':>10} {'bf16':>10} {'fp32':>10}")
     for C, F in ((320, 16), (1280, 24)):
