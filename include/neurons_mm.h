@@ -55,11 +55,22 @@ typedef enum nmm_dtype {
     NMM_F32 = 0,                /* parity mode: fp32 storage, fp32 FMA arithmetic (bar: max-abs 1e-4) */
     NMM_BF16 = 1,               /* production mode: bf16 storage + tcgen05 bf16 MMA, fp32 accumulate,
                                    fp32 residual stream, norms / softmax in fp32 (bar: max-abs 2e-2)  */
-    NMM_F32X3 = 2               /* fp32 storage (x, y, source parameters: float), fp32-grade arithmetic on the tensor cores:
+    NMM_F32X3 = 2,              /* fp32 storage (x, y, source parameters: float), fp32-grade arithmetic on the tensor cores:
                                    every Linear runs as three bf16 tcgen05 MMAs per product -- hi.hi + hi.lo + lo.hi of
                                    the two-term bf16 splits of both operands, fp32 accumulation in TMEM (bar: max-abs 1e-4,
                                    like NMM_F32, which stays as the FMA-pipe checker).  Needs channels % 64 == 0.
                                    nmm_shape.dtype only; nmm_params.dtype stays the source element type.              */
+    NMM_F32X6 = 3               /* fp32 storage (x, y, source parameters: float), fp32-exact arithmetic on the tensor cores:
+                                   GEMM operands are bf16 [rows, 3K] = hi | mid | lo planes (hi = bf16(v), mid = bf16(v - hi),
+                                   lo = bf16(v - hi - mid): ~24 significant bits), every Linear runs as six bf16 tcgen05 MMAs per
+                                   product -- the cross products of weight >= 2^-16 (lo.hi, mid.mid, hi.lo, mid.hi, hi.mid,
+                                   hi.hi; the dropped terms are <= 2^-24 relative), fp32 accumulation in TMEM restarted every
+                                   K = 320 with the partial sums added in fp32 by the epilogue; the spatial attention likewise
+                                   (six mma.sync products for S and for O, each 32-key tile's P.V folded into O in fp32).  Measured
+                                   (B200): GEMM error flat in K (1.5-2e-6 on N(0,1) outputs up to K = 5120, FMA GEMM 3.9e-6 ..
+                                   1.6e-5); attention 1.5-3e-5 against fp64 at max |logit| 60 like the FMA kernels (x3: 2-2.7e-4),
+                                   up to 2.7x the FMA kernels' error at smaller logits; module outputs within 2x of NMM_F32.  Needs channels % 64 == 0 (and ctx_dim % 64 == 0 for the spatial
+                                   transformer).  nmm_shape.dtype only; nmm_params.dtype stays the source element type.       */
 } nmm_dtype;
 
 /* Shape + hyper-parameters of one module call.  Mirrors the arguments that reach
@@ -313,7 +324,8 @@ NMM_API int nmm_spatial_forward_stats(const nmm_spatial_shape *s, const void *x,
  * i / kv_div (kv_div = frames for the text cross-attention, 1 for self-attention); o like q.  dtype NMM_BF16 (tensor cores; 16-byte
  * aligned, strides % 8 == 0), NMM_F32 (fp32 checker kernel) or NMM_F32X3 (fp32-grade, 3 bf16 MMAs per product): q, k, v are then
  * bf16 rows of a hi plane and a lo plane, the lo plane half a row stride after the hi plane (e.g. q rows [hi q | lo q], k | v rows
- * [hi k | hi v | lo k | lo v]), o is fp32.  head_dim in {40, 80, 160}. */
+ * [hi k | hi v | lo k | lo v]), o is fp32.  NMM_F32X6 (fp32-exact, 6 bf16 MMAs per product): q, k, v are bf16 rows of hi | mid | lo planes,
+ * each plane a third of a row stride after the previous one; o is fp32.  head_dim in {40, 80, 160}. */
 NMM_API int nmm_spatial_attention(int32_t dtype, const void *q, const void *k, const void *v, void *o, int64_t q_row_stride, int64_t kv_row_stride,
                                   int64_t o_row_stride, int64_t q_image_stride, int64_t kv_image_stride, int64_t o_image_stride, int32_t q_len,
                                   int32_t kv_len, int32_t heads, int32_t head_dim, int32_t images, int32_t kv_div, void *stream);

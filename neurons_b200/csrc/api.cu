@@ -114,7 +114,7 @@ static PackedLayout packed_layout(const Geo &g) {
     PackedLayout L;
     memset(&L, 0, sizeof(L));
     size_t off = 0;
-    const size_t C = g.C, ws = dtype_size(g.dtype);
+    const size_t C = g.C, ws = operand_size(g.dtype);
     auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
     L.header = take(sizeof(PackedHeader));
     L.gn_w = take(C * 4); L.gn_b = take(C * 4);
@@ -171,7 +171,8 @@ struct WorkLayout { size_t gn_partial, tok, tok2, h, big, ctx, ln_part, stat_par
 static WorkLayout work_layout(const Geo &g) {
     WorkLayout w;
     size_t off = 0;
-    const size_t es = dtype_size(g.dtype), NC = (size_t)g.B * g.F * chunk_positions(g) * g.C;     // one chunk
+    // es: bytes per GEMM-operand element (NMM_F32X6: three bf16 planes); the fp32 q | k | v of the fp32-grade modes fit in `big` (12 <= 4 es)
+    const size_t es = operand_size(g.dtype), NC = (size_t)g.B * g.F * chunk_positions(g) * g.C;     // one chunk
     auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 1024); return o; };
     w.gn_partial = take(gn_partial_bytes(g));
     w.tok = take(NC * es);          // GroupNorm tokens / LayerNorm output / GEMM-dtype copy of h for proj_out
@@ -192,9 +193,11 @@ static int validate(const nmm_shape *s) {
     if (!s) return fail(NMM_ERR_BAD_ARG, "shape is NULL");
     if (s->batch <= 0 || s->channels <= 0 || s->frames <= 0 || s->height <= 0 || s->width <= 0)
         return fail(NMM_ERR_BAD_ARG, "non-positive dimension");
-    if (s->dtype != NMM_F32 && s->dtype != NMM_BF16 && s->dtype != NMM_F32X3) return fail(NMM_ERR_BAD_ARG, "unknown dtype %d", s->dtype);
+    if (s->dtype != NMM_F32 && s->dtype != NMM_BF16 && s->dtype != NMM_F32X3 && s->dtype != NMM_F32X6) return fail(NMM_ERR_BAD_ARG, "unknown dtype %d", s->dtype);
     if (s->dtype == NMM_F32X3 && s->channels % 64 != 0)
         return fail(NMM_ERR_UNSUPPORTED, "NMM_F32X3 (3 x bf16 tensor-core mode) needs channels %% 64 == 0 (got %d); use NMM_F32", s->channels);
+    if (s->dtype == NMM_F32X6 && s->channels % 64 != 0)
+        return fail(NMM_ERR_UNSUPPORTED, "NMM_F32X6 (6 x bf16 tensor-core mode) needs channels %% 64 == 0 (got %d); use NMM_F32", s->channels);
     if (s->channels % NMM_GN_GROUPS != 0) return fail(NMM_ERR_BAD_ARG, "channels (%d) must be divisible by %d GroupNorm groups", s->channels, NMM_GN_GROUPS);
     if (s->heads <= 0 || s->channels % s->heads != 0) return fail(NMM_ERR_BAD_ARG, "channels (%d) must be divisible by heads (%d)", s->channels, s->heads);
     if (s->layers <= 0 || s->layers > NMM_MAX_LAYERS) return fail(NMM_ERR_UNSUPPORTED, "num_transformer_block %d outside [1,%d]", s->layers, NMM_MAX_LAYERS);
@@ -237,15 +240,16 @@ __global__ void convert_rows_kernel(const TS *__restrict__ src, TD *__restrict__
     }
 }
 
-// NMM_F32X3 weights: dst is bf16 [rows, 2 * cols], row r = hi plane | lo plane of src row map(r)  (w = hi + lo + O(2^-17 w))
-template <typename TS>
+// NMM_F32X3 weights: dst is bf16 [rows, 2 * cols], row r = hi plane | lo plane of src row map(r)  (w = hi + lo + O(2^-17 w));
+// NMM_F32X6 (PL 3): bf16 [rows, 3 * cols], hi | mid | lo planes (w = hi + mid + lo + O(2^-24 w))
+template <typename TS, int PL = 2>
 __global__ void split_rows_kernel(const TS *__restrict__ src, bf16 *__restrict__ dst, int64_t rows, int64_t cols, int64_t half) {
     pdl_wait();
     pdl_launch_dependents();
     const int64_t total = rows * cols;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
         const int64_t r = i / cols, c = i - r * cols;
-        split1_store(dst + r * 2 * cols, (int)cols, (int)c, to_f32(src[geglu_src_row(r, half) * cols + c]));
+        split1_store<PL>(dst + r * PL * cols, (int)cols, (int)c, to_f32(src[geglu_src_row(r, half) * cols + c]));
     }
 }
 
@@ -255,10 +259,17 @@ int launch_convert_rows(const void *src, int src_dtype, void *dst, int dst_dtype
     if (total == 0) return NMM_OK;
     const int threads = 256;
     const int blocks = (int)std::min<int64_t>(ceil_div(total, threads), 148 * 16);
-    ProfScope prof(K_PACK, st, 0.0, (double)total * (dtype_size(src_dtype) + dtype_size(dst_dtype)));
+    ProfScope prof(K_PACK, st, 0.0, (double)total * (dtype_size(src_dtype) + operand_size(dst_dtype)));
     if (dst_dtype == NMM_F32X3) {
         if (src_dtype == NMM_F32) launch_pdl(split_rows_kernel<float>, blocks, threads, 0, st, (const float *)src, (bf16 *)dst, rows, cols, (int64_t)half);
         else if (src_dtype == NMM_BF16) launch_pdl(split_rows_kernel<bf16>, blocks, threads, 0, st, (const bf16 *)src, (bf16 *)dst, rows, cols, (int64_t)half);
+        else return fail(NMM_ERR_BAD_ARG, "unknown parameter dtype");
+        NMM_LAUNCHED("split_rows_kernel");
+        return NMM_OK;
+    }
+    if (dst_dtype == NMM_F32X6) {
+        if (src_dtype == NMM_F32) launch_pdl(split_rows_kernel<float, 3>, blocks, threads, 0, st, (const float *)src, (bf16 *)dst, rows, cols, (int64_t)half);
+        else if (src_dtype == NMM_BF16) launch_pdl(split_rows_kernel<bf16, 3>, blocks, threads, 0, st, (const bf16 *)src, (bf16 *)dst, rows, cols, (int64_t)half);
         else return fail(NMM_ERR_BAD_ARG, "unknown parameter dtype");
         NMM_LAUNCHED("split_rows_kernel");
         return NMM_OK;
@@ -435,9 +446,9 @@ __global__ void make_pe_kernel(float *__restrict__ pe, int max_len, int C) {
 }
 
 static int linear(const Geo &g, const LinearArgs &a, cudaStream_t st) {
-    if (g.dtype == NMM_F32X3) {          // fp32-grade on the tensor cores: operands are hi | lo bf16 planes (gemm_tcgen05.cu, X3)
+    if (g.dtype == NMM_F32X3 || g.dtype == NMM_F32X6) {      // fp32-grade / fp32-exact on the tensor cores: operands are bf16 planes (gemm_tcgen05.cu, PL)
         LinearArgs b = a;
-        b.x3 = 1;
+        b.planes = planes_of(g.dtype);
         return launch_linear_tc(b, st);
     }
     return g.dtype == NMM_BF16 ? launch_linear_tc(a, st) : launch_linear_simt(a, st);
@@ -549,7 +560,7 @@ int nmm_pack_params(const nmm_shape *s, const nmm_params *src, void *packed, siz
             const nmm_attn_params &ap = lp.attn[i];
             const AttnOff &ao = lo.attn[i];
             PACK(ap.norm_w, ao.ln_w, NMM_F32, C, 1, 0); PACK(ap.norm_b, ao.ln_b, NMM_F32, C, 1, 0);
-            const size_t wbytes = (size_t)C * C * dtype_size(wd);
+            const size_t wbytes = (size_t)C * C * operand_size(wd);
             PACK(ap.to_out_w, ao.wo, wd, C, C, 0); PACK(ap.to_out_b, ao.bo, NMM_F32, C, 1, 0);
             if (g.pos_enc) {
                 if (ap.pe) PACK(ap.pe, ao.pe, NMM_F32, (int64_t)g.max_len, C, 0);
@@ -798,7 +809,7 @@ static int forward_impl(const nmm_shape *s, const void *x, void *y, const void *
                 if (attn_fused) {
                     a.epilogue = NMM_EPI_QKV_ATTN; a.W = pk + ao.wqkv_t; a.out = ctx; a.attn_B = g.B; a.attn_heads = g.heads;
                 }
-                if (g.dtype == NMM_F32X3) { a.h = (float *)big; a.out = nullptr; }      // q|k|v stay fp32 for the fp32 attention kernel
+                if (planes_of(g.dtype) > 1) { a.h = (float *)big; a.out = nullptr; }      // q|k|v stay fp32 for the fp32 attention kernel
                 if ((rc = linear(g, a, st)) != NMM_OK) return rc;
                 clear_fold(a);
                 // softmax(q k^T / sqrt(dh)) v over frames                               motion_module_new.py:258-287
@@ -986,7 +997,7 @@ int nmm_qkv_attention(const nmm_shape *s, const void *tokens, const void *wqkv, 
 
 int nmm_linear(int32_t dtype, int32_t epilogue, int64_t M, int32_t N, int32_t K, const void *A, const void *W, const float *bias,
                float *h, void *out, const nmm_shape *s, const void *x, void *y, void *stream) {
-    if (dtype != NMM_F32 && dtype != NMM_BF16 && dtype != NMM_F32X3) return fail(NMM_ERR_BAD_ARG, "unknown dtype %d", dtype);
+    if (dtype != NMM_F32 && dtype != NMM_BF16 && dtype != NMM_F32X3 && dtype != NMM_F32X6) return fail(NMM_ERR_BAD_ARG, "unknown dtype %d", dtype);
     if (!A || !W || M < 0 || N <= 0 || K <= 0) return fail(NMM_ERR_BAD_ARG, "bad GEMM arguments");
     int rc = device_check();
     if (rc != NMM_OK) return rc;
@@ -1012,7 +1023,7 @@ int nmm_linear(int32_t dtype, int32_t epilogue, int64_t M, int32_t N, int32_t K,
         }
         default: return fail(NMM_ERR_BAD_ARG, "unknown epilogue %d", epilogue);
     }
-    a.x3 = dtype == NMM_F32X3 ? 1 : 0;      // A / W / out are bf16 hi | lo plane tensors ([rows, 2K] / [M, 2N]); x, y fp32
+    a.planes = planes_of(dtype);      // NMM_F32X3 / X6: A / W / out are bf16 plane tensors ([rows, 2K | 3K] / [M, 2N | 3N]); x, y fp32
     return dtype == NMM_F32 ? launch_linear_simt(a, (cudaStream_t)stream) : launch_linear_tc(a, (cudaStream_t)stream);
 }
 

@@ -162,15 +162,19 @@ __global__ void __launch_bounds__(256) temporal_attention_kernel(const T *__rest
             const int f2 = r / npos, pl2 = r - f2 * npos;
             const T *src_row = sm + (pl2 * F + f2) * pitch;
             if constexpr (sizeof(T) == 4) {
-                if (split_out) {                      // NMM_F32X3: ctx is the next GEMM's A operand, bf16 [N, 2C] hi | lo planes
-                    bf16 *srow = reinterpret_cast<bf16 *>(ctx) + ((int64_t)(b * F + f2) * P + p0 + pl2) * (2 * C);
+                if (split_out) {                      // NMM_F32X3 / X6: ctx is the next GEMM's A operand, bf16 [N, 2C / 3C] hi | lo (| mid | lo) planes
+                    bf16 *srow = reinterpret_cast<bf16 *>(ctx) + ((int64_t)(b * F + f2) * P + p0 + pl2) * (split_out * C);
                     if (VEC > 1) {
                         for (int v = lane; v < W / 4; v += 32) {
                             const float4 f4 = *reinterpret_cast<const float4 *>(src_row + v * 4);
-                            split4_store(srow, C, c_off + v * 4, f4.x, f4.y, f4.z, f4.w);
+                            if (split_out == 3) split4_store<3>(srow, C, c_off + v * 4, f4.x, f4.y, f4.z, f4.w);
+                            else split4_store(srow, C, c_off + v * 4, f4.x, f4.y, f4.z, f4.w);
                         }
                     } else {
-                        for (int e = lane; e < W; e += 32) split1_store(srow, C, c_off + e, to_f32(src_row[e]));
+                        for (int e = lane; e < W; e += 32) {
+                            if (split_out == 3) split1_store<3>(srow, C, c_off + e, to_f32(src_row[e]));
+                            else split1_store(srow, C, c_off + e, to_f32(src_row[e]));
+                        }
                     }
                     continue;
                 }
@@ -523,7 +527,7 @@ int launch_temporal_attention(const Geo &g, const void *qkv, void *ctx, cudaStre
         if (g.dh % 8 == 0 && al) return launch_attn_t<bf16, 8>(g, (const bf16 *)qkv, (bf16 *)ctx, st);
         return launch_attn_t<bf16, 1>(g, (const bf16 *)qkv, (bf16 *)ctx, st);
     }
-    const int split = g.dtype == NMM_F32X3 ? 1 : 0;      // the context feeds to_out's tensor-core GEMM: hi | lo bf16 planes
+    const int split = planes_of(g.dtype) > 1 ? planes_of(g.dtype) : 0;      // the context feeds to_out's tensor-core GEMM: 2 / 3 bf16 planes
     if (g.dh % 4 == 0 && al && g.C % 4 == 0) return launch_attn_t<float, 4>(g, (const float *)qkv, (float *)ctx, st, split);
     return launch_attn_t<float, 1>(g, (const float *)qkv, (float *)ctx, st, split);
 }

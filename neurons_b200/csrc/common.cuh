@@ -115,7 +115,10 @@ inline Geo geo_of(const nmm_shape *s) {
     g.ln_fold = s->ln_fold != 0 && s->dtype == NMM_BF16;
     return g;
 }
-inline size_t dtype_size(int dtype) { return dtype == NMM_BF16 ? 2 : 4; }      // NMM_F32 and NMM_F32X3 store fp32
+inline size_t dtype_size(int dtype) { return dtype == NMM_BF16 ? 2 : 4; }      // NMM_F32, NMM_F32X3 and NMM_F32X6 store fp32
+// bf16 planes of a tensor-core GEMM operand (NMM_F32X3: hi | lo, NMM_F32X6: hi | mid | lo) and the operand's bytes per element
+inline int planes_of(int dtype) { return dtype == NMM_F32X3 ? 2 : dtype == NMM_F32X6 ? 3 : 1; }
+inline size_t operand_size(int dtype) { return dtype == NMM_F32X6 ? 6 : dtype_size(dtype); }
 
 // ---- device helpers ------------------------------------------------------------------------------
 __device__ __forceinline__ float warp_sum(float v) {
@@ -161,17 +164,40 @@ __device__ __forceinline__ void split_bf16x2(float x, float y, uint32_t &hi, uin
     hi = pack_bf16x2(x, y);
     lo = pack_bf16x2(x - bf16_lo(hi), y - bf16_hi(hi));
 }
-__device__ __forceinline__ void split4_store(bf16 *row, int K, int c, float a, float b, float cc, float d) {      // c % 4 == 0, row 8-byte aligned, K % 4 == 0
-    uint32_t h0, l0, h1, l1;
-    split_bf16x2(a, b, h0, l0);
-    split_bf16x2(cc, d, h1, l1);
-    *reinterpret_cast<uint2 *>(row + c) = make_uint2(h0, h1);
-    *reinterpret_cast<uint2 *>(row + K + c) = make_uint2(l0, l1);
+// NMM_F32X6 operand format: three bf16 terms, hi = bf16(v), mid = bf16(v - hi), lo = bf16(v - hi - mid) (both differences exact in fp32),
+// v = hi + mid + lo + O(2^-24 |v|).  A [rows, K] operand is a bf16 [rows, 3K] tensor: row r = hi plane | mid plane | lo plane.
+__device__ __forceinline__ void split3_bf16x2(float x, float y, uint32_t &hi, uint32_t &mid, uint32_t &lo) {
+    hi = pack_bf16x2(x, y);
+    const float rx = x - bf16_lo(hi), ry = y - bf16_hi(hi);
+    mid = pack_bf16x2(rx, ry);
+    lo = pack_bf16x2(rx - bf16_lo(mid), ry - bf16_hi(mid));
 }
+// PL = 2 (NMM_F32X3) or 3 (NMM_F32X6) planes of K values per row
+template <int PL = 2>
+__device__ __forceinline__ void split4_store(bf16 *row, int K, int c, float a, float b, float cc, float d) {      // c % 4 == 0, row 8-byte aligned, K % 4 == 0
+    if constexpr (PL == 3) {
+        uint32_t h0, m0, l0, h1, m1, l1;
+        split3_bf16x2(a, b, h0, m0, l0);
+        split3_bf16x2(cc, d, h1, m1, l1);
+        *reinterpret_cast<uint2 *>(row + c) = make_uint2(h0, h1);
+        *reinterpret_cast<uint2 *>(row + K + c) = make_uint2(m0, m1);
+        *reinterpret_cast<uint2 *>(row + 2 * K + c) = make_uint2(l0, l1);
+    } else {
+        uint32_t h0, l0, h1, l1;
+        split_bf16x2(a, b, h0, l0);
+        split_bf16x2(cc, d, h1, l1);
+        *reinterpret_cast<uint2 *>(row + c) = make_uint2(h0, h1);
+        *reinterpret_cast<uint2 *>(row + K + c) = make_uint2(l0, l1);
+    }
+}
+template <int PL = 2>
 __device__ __forceinline__ void split1_store(bf16 *row, int K, int c, float v) {
     const bf16 h = __float2bfloat16_rn(v);
     row[c] = h;
-    row[K + c] = __float2bfloat16_rn(v - __bfloat162float(h));
+    const float r = v - __bfloat162float(h);
+    const bf16 m = __float2bfloat16_rn(r);
+    row[K + c] = m;
+    if constexpr (PL == 3) row[2 * K + c] = __float2bfloat16_rn(r - __bfloat162float(m));
 }
 
 // exact (erf) GELU, as torch.nn.functional.gelu default -- motion_module_new.py:510-518
@@ -250,7 +276,7 @@ int launch_y_sums_tiles(const float2 *part, double *sums, int B, int F, int tile
 int launch_y_sums_channels(const float2 *part, double *sums, int BF, int C, int P, cudaStream_t st);
 int launch_gn_partial_to_sums(const Geo &g, const double *partial, double *sums, cudaStream_t st);
 int launch_gn_tokens(const Geo &g, const nmm_shape *s, const Geo &full, const void *x, const double *partial, const float *gn_w,
-                     const float *gn_b, void *tokens, cudaStream_t st, int splits_override = 0);      // NMM_F32X3: tokens = bf16 [N, 2C] hi | lo planes
+                     const float *gn_b, void *tokens, cudaStream_t st, int splits_override = 0);      // NMM_F32X3 / X6: tokens = bf16 [N, 2C / 3C] planes
 // LayerNorm (+PE)
 int launch_layernorm_pe(const Geo &g, const nmm_shape *s, const float *h, const float *w, const float *b,
                         const float *pe, void *out, cudaStream_t st);
@@ -263,7 +289,7 @@ struct FlashArgs {
     void *o;
     int64_t q_rs, kv_rs, o_rs;      // row strides (elements)
     int64_t q_bs, kv_bs, o_bs;      // image strides (elements); the k / v image of q image i is i / kv_div
-    int64_t q_lo_off, kv_lo_off;    // launch_spatial_attention_x3 only: element offset of the lo plane inside a q / k-v row (hi | lo planes)
+    int64_t q_lo_off, kv_lo_off;    // launch_spatial_attention_x3 / _x6 only: element offset from one bf16 plane to the next inside a q / k-v row
     int Lq, Lkv, heads, images, kv_div, dh;
     int dtype;                      // NMM_BF16 (mma.sync flash kernel) or NMM_F32 (fp32 kernels: tiled FMA-pipe flash or checker)
     float scale, scale_log2e;       // dh^-1/2 and dh^-1/2 * log2(e)
@@ -272,6 +298,7 @@ int launch_spatial_attention(const FlashArgs &a, cudaStream_t st);
 bool spatial_attention_tc_eligible(const FlashArgs &a);                            // spatial_attention_tc.cu (tcgen05 / TMEM / TMA)
 int launch_spatial_attention_tc(const FlashArgs &a, int variant, cudaStream_t st);
 int launch_spatial_attention_x3(const FlashArgs &a, cudaStream_t st);               // spatial_attention_x3.cu: fp32-grade (hi | lo bf16 planes in, fp32 out)
+int launch_spatial_attention_x6(const FlashArgs &a, cudaStream_t st);               // spatial_attention_x6.cu: fp32-exact (hi | mid | lo bf16 planes in, fp32 out)
 bool spatial_attention_f32_tiled_eligible(const FlashArgs &a);                      // spatial_attention_f32.cu: NMM_F32 flash kernel on the FMA pipe
 int launch_spatial_attention_f32_tiled(const FlashArgs &a, cudaStream_t st);
 int device_check();
@@ -292,8 +319,9 @@ struct LinearArgs {
     float *h;                // RESIDUAL: fp32 [M,N] in/out
     void *out;               // STORE: [M,N]; RESIDUAL: optional [M,N] copy; GEGLU: [M,N/2]   (dtype)
     int no_h_store;          // RESIDUAL: h is only read, the sum goes to `out` alone (the last feed-forward)
-    int x3;                  // NMM_F32X3 (tensor-core path only): A is bf16 [M, 2K] and W bf16 [N, 2K], each row = hi plane | lo plane; `out`
-                             // is written the same way ([M, 2N], GEGLU [M, N]); x / y of the OUTPUT epilogue are fp32 (gemm_tcgen05.cu, X3)
+    int planes;              // 0 / 1: plain bf16.  2 (NMM_F32X3) / 3 (NMM_F32X6), tensor-core path only: A is bf16 [M, planes * K] and W bf16
+                             // [N, planes * K], each row = hi | lo (| mid | lo) planes; `out` is written the same way ([M, planes * N], GEGLU
+                             // [M, planes * N / 2]); x / y of the OUTPUT epilogue are fp32 (gemm_tcgen05.cu, PL)
     // OUTPUT epilogue
     const void *x; void *y;
     int F, P;
@@ -366,7 +394,7 @@ bool fused_module_eligible(const Geo &g, const nmm_shape *s, const void *x);
 int launch_fused_module(const FusedArgs &a, cudaStream_t st);
 int launch_linear_simt(const LinearArgs &a, cudaStream_t st);     // fp32
 int launch_linear_tc(const LinearArgs &a, cudaStream_t st);       // bf16 tcgen05
-int linear_dispatch(int dtype, const LinearArgs &a, cudaStream_t st);     // bf16 -> tcgen05, NMM_F32X3 -> tcgen05 3 x bf16, NMM_F32 -> FMA
+int linear_dispatch(int dtype, const LinearArgs &a, cudaStream_t st);     // bf16 -> tcgen05, NMM_F32X3 / X6 -> tcgen05 3 / 6 x bf16, NMM_F32 -> FMA
 // parameter packing
 int launch_convert_rows(const void *src, int src_dtype, void *dst, int dst_dtype, int64_t rows, int64_t cols,
                         int interleave_half /*0 or rows/2*/, cudaStream_t st);

@@ -32,7 +32,7 @@ struct EpiParams {
 
 // OUTPUT epilogue: can the bf16 16-byte vector path run (and with it the y-statistics emission)?
 inline bool output_vec_ok(const LinearArgs &a) {
-    return a.epilogue == NMM_EPI_OUTPUT && !a.x3 && a.P > 0 && a.P % 32 == 0 && aligned(a.x, 16) && aligned(a.y, 16) && a.xsb % 8 == 0 &&
+    return a.epilogue == NMM_EPI_OUTPUT && a.planes <= 1 && a.P > 0 && a.P % 32 == 0 && aligned(a.x, 16) && aligned(a.y, 16) && a.xsb % 8 == 0 &&
            a.xsc % 8 == 0 && a.xsf % 8 == 0 && a.ysb % 8 == 0 && a.ysc % 8 == 0 && a.ysf % 8 == 0;
 }
 

@@ -71,7 +71,10 @@ struct TcParams {
     int epi_buf;             // bytes of shared memory per epilogue warp (8 KB; 12 KB when a residual epilogue also writes a bf16 copy)
     unsigned long long *trace;   // NMM_TRACE builds only: per-tile timestamps of CTA 0 (development instrumentation)
     int debug;               // NMM_GEMM_DEBUG (timing experiments only, results invalid): 1 = epilogue does nothing, 2 = no TMA loads
+    int chunk_kb;            // PL 3: k-blocks per accumulator chunk (the epilogue sums the chunks in fp32 registers); otherwise unused
 };
+constexpr int TC_X6_CHUNK_KB = 5;      // PL 3: K = 320 per TMEM accumulator chunk
+constexpr int TC_X6_MAX_BN = 128;      // PL 3: the epilogue holds 2 x 32 columns of chunk sums per thread
 
 // GroupNorm-fused A operand (GNA instantiation): where the statistics and affine parameters live, and the x geometry
 struct GnParams {
@@ -186,10 +189,19 @@ __device__ __forceinline__ void fused_attention_phase(const AttnParams &at, uint
 // LNF: LayerNorm-folding roles compiled in (consumer transform / producer statistics).  Kept out of the default instantiation:
 // a run-time branch inside the unrolled epilogue loops costs the GEGLU epilogue its instruction-level parallelism (measured
 // 128 -> 204 us at C = 320).
-// X3: fp32-grade mode (NMM_F32X3).  Both operands arrive as bf16 [rows, 2K] = [hi | lo] planes (v = hi + lo + O(2^-17 v)); the K loop runs
+// PL: bf16 planes per operand.  1 = plain bf16.
+// PL = 2, fp32-grade mode (NMM_F32X3).  Both operands arrive as bf16 [rows, 2K] = [hi | lo] planes (v = hi + lo + O(2^-17 v)); the K loop runs
 // 3 * K / 64 k-blocks: hi.hi, hi.lo and lo.hi products accumulated in fp32 (the lo.lo term, 2^-16 relative, is dropped) -- the same
 // mainloop, three passes over the planes.  GEMM-operand outputs (`out`) are written as hi | lo planes too; x / y of the OUTPUT epilogue are fp32.
-template <int EPI, int CG, bool LNF, bool GNA, bool X3>
+// PL = 3, fp32-exact mode (NMM_F32X6).  Operands are bf16 [rows, 3K] = [hi | mid | lo] planes (v = hi + mid + lo + O(2^-24 v)); the K loop
+// runs 6 * K / 64 k-blocks, one pass per product of weight >= 2^-16, SMALL TERMS FIRST: lo.hi, mid.mid, hi.lo (2^-16), mid.hi, hi.mid (2^-8),
+// hi.hi (the dropped mid.lo, lo.mid, lo.lo are <= 2^-24).  The tensor core's fp32 accumulation is not round-to-nearest: measured on a B200,
+// one accumulator over the whole k-block sequence gave an error that grows about linearly with K (3.8e-5 at K = 5120 on N(0, 1) outputs,
+// 2.4x the FMA GEMM's).  So the sequence runs in chunks of p.chunk_kb k-blocks (K = 320), each into a fresh accumulator of the two TMEM
+// buffers; the epilogue warps add the chunk results in fp32 registers (round to nearest) while the next chunk accumulates, write the sum back
+// into the last chunk's accumulator and drain that as usual.  Small terms first keeps the small passes' roundings at their own magnitude
+// (tests/test_fp32_exact_tc.py emulates both orders).  `out` is written as hi | mid | lo planes; fp32 outputs stay fp32.
+template <int EPI, int CG, bool LNF, bool GNA, int PL>
 __global__ void __launch_bounds__(EPI == NMM_EPI_QKV_ATTN ? TC_THREADS + 32 * TC_ATTN_HELPERS : GNA ? TC_THREADS + 32 * TC_GN_WARPS : TC_THREADS, 1)
 linear_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_w,
                  const __grid_constant__ CUtensorMap tm_h,      // fp32 [M,N], box 32 x 32, 128-byte swizzle (residual load / h store)
@@ -216,10 +228,19 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int nk = (p.K + TC_BK - 1) / TC_BK;                        // k-blocks of one operand plane
-    const int num_kb = X3 ? 3 * nk : nk;
-    // X3: k-block kb = pass t * nk + j multiplies A plane (t == 2 ? lo : hi) by W plane (t == 1 ? lo : hi); small terms last
-    auto a_col = [&](int kb) { if constexpr (X3) { const int t = kb / nk, j = kb - t * nk; return (t == 2 ? nk + j : j) * TC_BK; } else return kb * TC_BK; };
-    auto w_col = [&](int kb) { if constexpr (X3) { const int t = kb / nk, j = kb - t * nk; return (t == 1 ? nk + j : j) * TC_BK; } else return kb * TC_BK; };
+    const int num_kb = PL == 3 ? 6 * nk : PL == 2 ? 3 * nk : nk;
+    // PL = 2: k-block kb = pass t * nk + j multiplies A plane (t == 2 ? lo : hi) by W plane (t == 1 ? lo : hi); small terms last.
+    // PL = 3: pass t multiplies A plane (0x46 >> 2t) & 3 by W plane (0x124 >> 2t) & 3 (plane 0 = hi, 1 = mid, 2 = lo): the order above.
+    auto a_col = [&](int kb) {
+        if constexpr (PL == 3) { const int t = kb / nk, j = kb - t * nk; return (((0x46 >> (2 * t)) & 3) * nk + j) * TC_BK; }
+        else if constexpr (PL == 2) { const int t = kb / nk, j = kb - t * nk; return (t == 2 ? nk + j : j) * TC_BK; }
+        else return kb * TC_BK;
+    };
+    auto w_col = [&](int kb) {
+        if constexpr (PL == 3) { const int t = kb / nk, j = kb - t * nk; return (((0x124 >> (2 * t)) & 3) * nk + j) * TC_BK; }
+        else if constexpr (PL == 2) { const int t = kb / nk, j = kb - t * nk; return (t == 1 ? nk + j : j) * TC_BK; }
+        else return kb * TC_BK;
+    };
     // Tile schedule: a cluster walks (m_group, n_blk) pairs; CTA `rank` of the cluster owns m-block m_group*CG + rank.
     // Both CTAs of a pair run the same number of iterations (a phantom m-block past the end is all zero-fill + clipped).
     // rank inside the (CG, 1, 1) cluster = blockIdx.x % CG, taken from blockIdx on purpose: the compiler must KNOW it is uniform.  With
@@ -362,8 +383,20 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                 ptx::mbar_wait(tempty_bar(as), aphase ^ 1u);           // every epilogue warp (of both CTAs) drained this accumulator
                 TRACE(tile_no, 1);
                 ptx::tc_fence_after();
-                const uint32_t d_tmem = tmem_base + (uint32_t)(as * p.block_n);
+                uint32_t d_tmem = tmem_base + (uint32_t)(as * p.block_n);
                 for (int kb = 0; kb < num_kb; kb++) {
+                    int kc = kb;                                              // k-block index inside the current accumulator
+                    if constexpr (PL == 3) {
+                        kc = kb % p.chunk_kb;
+                        if (kc == 0 && kb > 0) {                              // chunk boundary: publish this accumulator, go on in the other buffer
+                            if (ptx::elect_one()) ptx::umma_commit<CG>(tfull_bar(as));
+                            __syncwarp();
+                            if (++as == 2) { as = 0; aphase ^= 1u; }
+                            ptx::mbar_wait(tempty_bar(as), aphase ^ 1u);
+                            ptx::tc_fence_after();
+                            d_tmem = tmem_base + (uint32_t)(as * p.block_n);
+                        }
+                    }
                     // TMA bytes (of both CTAs) have landed; GNA: ... and the converter warps have normalised the A tile
                     ptx::mbar_wait(GNA ? conv_bar(stage) : full_bar(stage), phase);
                     if (kb == 0) TRACE(tile_no, 2);
@@ -391,13 +424,13 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                             const uint64_t b_desc2 = ptx::umma_smem_desc_sw128(sa + TC_A_BYTES + (n_mma / CG) * TC_BK * 2);
 #pragma unroll
                             for (int k = 0; k < TC_BK / 16; k++) {
-                                ptx::umma_bf16<CG>(d_tmem, a_desc + (uint64_t)(k * 2), b_desc + (uint64_t)(k * 2), idesc, (kb | k) != 0 ? 1u : 0u);
-                                ptx::umma_bf16<CG>(d_tmem + n_mma, a_desc + (uint64_t)(k * 2), b_desc2 + (uint64_t)(k * 2), idesc, (kb | k) != 0 ? 1u : 0u);
+                                ptx::umma_bf16<CG>(d_tmem, a_desc + (uint64_t)(k * 2), b_desc + (uint64_t)(k * 2), idesc, (kc | k) != 0 ? 1u : 0u);
+                                ptx::umma_bf16<CG>(d_tmem + n_mma, a_desc + (uint64_t)(k * 2), b_desc2 + (uint64_t)(k * 2), idesc, (kc | k) != 0 ? 1u : 0u);
                             }
                         } else {
 #pragma unroll
                             for (int k = 0; k < TC_BK / 16; k++)         // +32 bytes per K=16 step inside the swizzle atom
-                                ptx::umma_bf16<CG>(d_tmem, a_desc + (uint64_t)(k * 2), b_desc + (uint64_t)(k * 2), idesc, (kb | k) != 0 ? 1u : 0u);
+                                ptx::umma_bf16<CG>(d_tmem, a_desc + (uint64_t)(k * 2), b_desc + (uint64_t)(k * 2), idesc, (kc | k) != 0 ? 1u : 0u);
                         }
                     }
                     ptx::umma_commit<CG>(empty_bar(stage));               // stage reusable (in both CTAs) once these MMAs retire
@@ -500,6 +533,55 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
             const int n_blk = (int)(ct - m_grp * p.n_tiles);
             const int64_t m_blk = m_grp * CG + rank;
             const int64_t row0 = m_blk * TC_BM + q * 32;
+            if constexpr (PL == 3) {
+                // the chunks of this tile (see PL above): every warp adds its columns of each chunk into fp32 running sums and releases the
+                // buffer; the last chunk's accumulator receives the sum and is drained below like any accumulator.  The sums (this lane's
+                // row, 64 columns) live in the warp's first two epilogue boxes, 16-byte slots XOR-rotated by lane (conflict-free)
+                const int nch = (num_kb + p.chunk_kb - 1) / p.chunk_kb;
+                const uint32_t box0c = epi_base + (uint32_t)ew * (uint32_t)p.epi_buf;
+                auto slot = [&](int v) { return box0c + (uint32_t)lane * 256u + (uint32_t)(((v ^ lane) & 15) << 4); };
+                if (lane == 0) ptx::bulk_wait_read0();                    // the previous tile's stores have read the boxes
+                __syncwarp();
+                for (int ch = 0; ch < nch; ch++) {
+                    ptx::mbar_wait(tfull_bar(as), aphase);
+                    ptx::tc_fence_after();
+                    const uint32_t tb = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(as * p.block_n);
+#pragma unroll
+                    for (int i = 0; i < 2; i++) {
+                        const int col = EPI == NMM_EPI_GEGLU ? half * 64 + 32 * i : half * 32 + 64 * i;     // the columns this warp drains below
+                        if (col < p.block_n) {
+                            uint32_t r[32];
+                            ptx::tmem_ld32(tb + (uint32_t)col, r);
+                            ptx::tmem_ld_wait();
+#pragma unroll
+                            for (int v = 0; v < 8; v++) {
+                                if (ch > 0) {
+                                    const float4 s4 = lds128(slot(8 * i + v));
+                                    r[4 * v] = __float_as_uint(s4.x + __uint_as_float(r[4 * v]));
+                                    r[4 * v + 1] = __float_as_uint(s4.y + __uint_as_float(r[4 * v + 1]));
+                                    r[4 * v + 2] = __float_as_uint(s4.z + __uint_as_float(r[4 * v + 2]));
+                                    r[4 * v + 3] = __float_as_uint(s4.w + __uint_as_float(r[4 * v + 3]));
+                                }
+                                if (ch < nch - 1) sts128(slot(8 * i + v), r[4 * v], r[4 * v + 1], r[4 * v + 2], r[4 * v + 3]);
+                            }
+                            if (ch == nch - 1) ptx::tmem_st32(tb + (uint32_t)col, r);
+                        }
+                    }
+                    if (ch == nch - 1) {
+                        ptx::tmem_st_wait();
+                        ptx::fence_proxy_async();                         // generic writes to the boxes before TMA reuses them
+                        __syncwarp();
+                        break;
+                    }
+                    ptx::tc_fence_before();
+                    __syncwarp();
+                    if (lane == 0) {
+                        if (CG == 1) ptx::mbar_arrive(tempty_bar(as));
+                        else ptx::mbar_arrive_cluster(tempty_bar(as) & ptx::PEER_MASK);
+                    }
+                    if (++as == 2) { as = 0; aphase ^= 1u; }
+                }
+            }
             const uint32_t t_row = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(as * p.block_n);
             if (warp == 4 && lane == 0) TRACE(tile_no, 6);
             float ln_mu = 0.f, ln_rstd = 0.f;
@@ -653,7 +735,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                                 float acc[16];
 #pragma unroll
                                 for (int j = 0; j < 16; j++) acc[j] = __uint_as_float(r[j]);
-                                epilogue_apply<EPI, std::conditional_t<X3, float, bf16>, 16>(e, row, col0, acc);
+                                epilogue_apply<EPI, std::conditional_t<(PL > 1), float, bf16>, 16>(e, row, col0, acc);
                             }
                         }
                     }
@@ -664,7 +746,8 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                     const int col0 = n_blk * p.block_n + c0;
                     wait_acc();
                     uint32_t o[16];
-                    uint32_t olo[X3 ? 16 : 1];                             // X3: bf16 residuals of the outputs (the lo plane)
+                    uint32_t olo[PL > 1 ? 16 : 1];                         // PL 2: bf16 residuals of the outputs (the lo plane); PL 3: the mid plane
+                    uint32_t olo2[PL == 3 ? 16 : 1];                       // PL 3: the lo plane
                     // both 32-column halves are requested before the single tcgen05.wait::ld: one exposed TMEM latency per chunk
                     uint32_t r[2][32];
                     ptx::tmem_ld32(t_row + (uint32_t)c0, r[0]);
@@ -697,7 +780,8 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                             }
                             float y0, y1;
                             geglu_pair(v0, g0, v1, g1, y0, y1);
-                            if constexpr (X3) split_bf16x2(y0, y1, o[8 * hc + j], olo[8 * hc + j]);
+                            if constexpr (PL == 3) split3_bf16x2(y0, y1, o[8 * hc + j], olo[8 * hc + j], olo2[8 * hc + j]);
+                            else if constexpr (PL == 2) split_bf16x2(y0, y1, o[8 * hc + j], olo[8 * hc + j]);
                             else o[8 * hc + j] = pack_bf16x2(y0, y1);
                         }
                     };
@@ -707,15 +791,20 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                     __syncwarp();
 #pragma unroll
                     for (int j = 0; j < 4; j++) sts128(box_bf16_addr(box0, lane, j), o[4 * j], o[4 * j + 1], o[4 * j + 2], o[4 * j + 3]);
-                    if constexpr (X3) {
+                    if constexpr (PL > 1) {
 #pragma unroll
                         for (int j = 0; j < 4; j++) sts128(box_bf16_addr(box1, lane, j), olo[4 * j], olo[4 * j + 1], olo[4 * j + 2], olo[4 * j + 3]);
+                    }
+                    if constexpr (PL == 3) {      // the third box of the 12 KB per-warp buffer (host: epi_buf)
+#pragma unroll
+                        for (int j = 0; j < 4; j++) sts128(box_bf16_addr(box2, lane, j), olo2[4 * j], olo2[4 * j + 1], olo2[4 * j + 2], olo2[4 * j + 3]);
                     }
                     ptx::fence_proxy_async();
                     __syncwarp();
                     if (lane == 0) {
                         ptx::tma_store_2d(&tm_o, box0, col0 / 2, (int32_t)row0);
-                        if constexpr (X3) ptx::tma_store_2d(&tm_o, box1, p.N / 2 + col0 / 2, (int32_t)row0);      // lo plane: columns [N/2, N) of `out`
+                        if constexpr (PL > 1) ptx::tma_store_2d(&tm_o, box1, p.N / 2 + col0 / 2, (int32_t)row0);      // lo (PL 3: mid) plane: columns [N/2, N) of `out`
+                        if constexpr (PL == 3) ptx::tma_store_2d(&tm_o, box2, p.N + col0 / 2, (int32_t)row0);         // PL 3: lo plane, columns [N, 3N/2)
                         ptx::bulk_commit();
                     }
                     if (warp == 4 && lane == 0 && c0 / 128 < 4) TRACE(tile_no, 8 + c0 / 128);
@@ -782,7 +871,7 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                             const float4 h4 = lds128(box_f32_addr(box, lane, j));
                             v[4 * j] += h4.x; v[4 * j + 1] += h4.y; v[4 * j + 2] += h4.z; v[4 * j + 3] += h4.w;
                         }
-                        if (e.out != nullptr && !e.no_h_store && lane == 0) ptx::bulk_wait_read0();   // third box (bf16 copy) free again
+                        if (e.out != nullptr && (PL == 3 || !e.no_h_store) && lane == 0) ptx::bulk_wait_read0();   // third box (bf16 copy; PL 3: lo plane) free again
                         __syncwarp();                                     // every lane has read its row before the box is overwritten
                     } else {
                         if (lane == 0) ptx::bulk_wait_read0();            // the previous chunk's boxes have been read
@@ -804,7 +893,17 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                                    __float_as_uint(v[4 * j + 3]));
                     }
                     if (want_o) {
-                        if constexpr (X3) {                               // hi plane -> obox, lo plane -> obox + 2 KB (both halves of a 4 KB box)
+                        if constexpr (PL == 3) {                          // hi plane -> obox, mid plane -> obox + 2 KB, lo plane -> box2 (host: epi_buf 12 KB)
+                            uint32_t hi[16], mid[16], lo[16];
+#pragma unroll
+                            for (int j = 0; j < 16; j++) split3_bf16x2(v[2 * j], v[2 * j + 1], hi[j], mid[j], lo[j]);
+#pragma unroll
+                            for (int j = 0; j < 4; j++) {
+                                sts128(box_bf16_addr(obox, lane, j), hi[4 * j], hi[4 * j + 1], hi[4 * j + 2], hi[4 * j + 3]);
+                                sts128(box_bf16_addr(obox + 2048u, lane, j), mid[4 * j], mid[4 * j + 1], mid[4 * j + 2], mid[4 * j + 3]);
+                                sts128(box_bf16_addr(box2, lane, j), lo[4 * j], lo[4 * j + 1], lo[4 * j + 2], lo[4 * j + 3]);
+                            }
+                        } else if constexpr (PL == 2) {                   // hi plane -> obox, lo plane -> obox + 2 KB (both halves of a 4 KB box)
                             uint32_t hi[16], lo[16];
 #pragma unroll
                             for (int j = 0; j < 16; j++) split_bf16x2(v[2 * j], v[2 * j + 1], hi[j], lo[j]);
@@ -825,7 +924,8 @@ linear_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
                     if (lane == 0) {
                         if (want_h) ptx::tma_store_2d(&tm_h, box, col0, (int32_t)row0);
                         if (want_o) ptx::tma_store_2d(&tm_o, obox, col0, (int32_t)row0);
-                        if constexpr (X3) { if (want_o) ptx::tma_store_2d(&tm_o, obox + 2048u, p.N + col0, (int32_t)row0); }   // lo plane: columns [N, 2N)
+                        if constexpr (PL > 1) { if (want_o) ptx::tma_store_2d(&tm_o, obox + 2048u, p.N + col0, (int32_t)row0); }   // lo (PL 3: mid) plane: columns [N, 2N)
+                        if constexpr (PL == 3) { if (want_o) ptx::tma_store_2d(&tm_o, box2, 2 * p.N + col0, (int32_t)row0); }      // PL 3: lo plane, columns [2N, 3N)
                         ptx::bulk_commit();
                     }
                     if (warp == 4 && lane == 0 && k < 4) TRACE(tile_no, 8 + k);
@@ -970,7 +1070,8 @@ static int num_sms() {                 // SM count of the CURRENT device (cached
 //   whole GEMM    ceil(cluster_tiles / resident clusters) * per tile            (wave quantisation)
 // The per-SM ingest of ~64 B/clk is why only (CG = 2, bn = 256) can keep the tensor pipe fully fed, and why small tiles lose.
 struct TilePlan { int block_n, cluster, wide; };
-static TilePlan choose_tiles(int64_t m_tiles, int N, int K, int sms, int gran, int force_cluster, int force_bn, bool allow_wide = false) {
+static TilePlan choose_tiles(int64_t m_tiles, int N, int K, int sms, int gran, int force_cluster, int force_bn, bool allow_wide = false,
+                             int max_bn = 256) {
     TilePlan best = {0, 1, 0};
     double best_cost = 1e300;
     const int num_kb = (K + TC_BK - 1) / TC_BK;
@@ -978,7 +1079,7 @@ static TilePlan choose_tiles(int64_t m_tiles, int N, int K, int sms, int gran, i
         if (force_cluster && cg != force_cluster) continue;
         if (cg == 2 && (m_tiles < 2 || sms % 2 != 0)) continue;
         const int64_t m_groups = ceil_div(m_tiles, cg);
-        for (int bn = 256; bn >= gran; bn -= gran) {
+        for (int bn = max_bn / gran * gran; bn >= gran; bn -= gran) {
             if (N % bn) continue;
             if (force_bn && bn != force_bn) continue;
             const double mma = 2.0 * bn, fill = (16384.0 + bn * 128.0 / cg) / 64.0;
@@ -1012,11 +1113,11 @@ void plan_linear_tc(int64_t M, int N, int K, int epilogue, int *block_n, int *cl
     *cluster = plan.cluster;
 }
 
-template <int EPI, int CG, bool LNF, bool GNA = false, bool X3 = false>
+template <int EPI, int CG, bool LNF, bool GNA = false, int PL = 1>
 static int launch_tc_t(const CUtensorMap &ta, const CUtensorMap &tw, const CUtensorMap &th, const CUtensorMap &to, const TcParams &p,
                        const EpiParams &e, size_t smem, int grid, cudaStream_t st, double flops, double bytes, const GnParams &gn = GnParams(),
                        const AttnParams &at = AttnParams()) {
-    auto kern = linear_tc_kernel<EPI, CG, LNF, GNA, X3>;
+    auto kern = linear_tc_kernel<EPI, CG, LNF, GNA, PL>;
     static DeviceOnce once;           // per template instantiation and device
     NMM_CUDA_OK(once.max_smem(kern, TC_SMEM_MAX));
     cudaLaunchConfig_t cfg;
@@ -1047,10 +1148,12 @@ int launch_linear_tc(const LinearArgs &a, cudaStream_t st) {
     if (a.N % 32 != 0) return fail(NMM_ERR_UNSUPPORTED, "tcgen05 GEMM needs N %% 32 == 0 (N=%d)", a.N);
     if (a.epilogue == NMM_EPI_GEGLU && a.N % 64 != 0) return fail(NMM_ERR_UNSUPPORTED, "GEGLU epilogue needs N %% 64 == 0 (N=%d)", a.N);
     if (a.K % 8 != 0) return fail(NMM_ERR_UNSUPPORTED, "tcgen05 GEMM needs K %% 8 == 0 (K=%d)", a.K);
-    const bool x3 = a.x3 != 0;
+    const int planes = a.planes > 1 ? a.planes : 1;
+    if (planes > 3) return fail(NMM_ERR_BAD_ARG, "tcgen05 GEMM: %d operand planes (1, 2 or 3)", planes);
+    const bool x3 = planes > 1;
     if (x3 && (a.K % TC_BK != 0 || a.gn_x != nullptr || a.epilogue == NMM_EPI_QKV_ATTN || a.ln_part_in != nullptr || a.ln_part_out != nullptr ||
                (a.epilogue == NMM_EPI_STORE && a.out != nullptr) || (a.epilogue == NMM_EPI_RESIDUAL && a.out != nullptr && !a.no_h_store)))
-        return fail(NMM_ERR_UNSUPPORTED, "3 x bf16 (fp32-grade) tensor-core GEMM: needs K %% 64 == 0, no fused GroupNorm / attention / LayerNorm folding, and a STORE epilogue writing fp32 only");
+        return fail(NMM_ERR_UNSUPPORTED, "3 / 6 x bf16 (fp32-grade / fp32-exact) tensor-core GEMM: needs K %% 64 == 0, no fused GroupNorm / attention / LayerNorm folding, and a STORE epilogue writing fp32 only");
     if (a.M <= 0) return NMM_OK;
     TcParams p;
     p.M = a.M; p.N = a.N; p.K = a.K;
@@ -1068,6 +1171,7 @@ int launch_linear_tc(const LinearArgs &a, cudaStream_t st) {
     const int force_bn = (int)opt(NMM_OPT_GEMM_BLOCK_N);
     p.debug = debug_flags;
     p.trace = nullptr;
+    p.chunk_kb = planes == 3 ? TC_X6_CHUNK_KB : 0;
 #ifdef NMM_TRACE
     if (!g_trace_dev) { cudaMalloc(&g_trace_dev, TRACE_TILES * TRACE_SLOTS * 8); cudaMemset(g_trace_dev, 0, TRACE_TILES * TRACE_SLOTS * 8); }
     p.trace = g_trace_dev;
@@ -1081,10 +1185,11 @@ int launch_linear_tc(const LinearArgs &a, cudaStream_t st) {
                 !linear_tc_gn_fusable(a.M, a.P, a.gn_x, a.xsb, a.xsc, a.xsf) || (int64_t)a.gn_B * a.F * a.P != a.M))
         return fail(NMM_ERR_UNSUPPORTED, "GroupNorm-fused A operand: needs the STORE epilogue, P %% 64 == 0, M %% 128 == 0 and 16-byte aligned x");
     const int gran = a.epilogue == NMM_EPI_GEGLU ? 64 : 32;
-    const bool allow_wide = a.epilogue == NMM_EPI_RESIDUAL && !gna && a.ln_part_in == nullptr && a.ln_part_out == nullptr && !(debug_flags & 2) && opt(NMM_OPT_WIDE_TILE) != 0;
+    const bool allow_wide = a.epilogue == NMM_EPI_RESIDUAL && planes != 3 && !gna && a.ln_part_in == nullptr && a.ln_part_out == nullptr && !(debug_flags & 2) && opt(NMM_OPT_WIDE_TILE) != 0;
     const TilePlan plan = attn ? TilePlan{3 * NMM_ATTN_TILE_CH, 1, 0} :
-                          choose_tiles(p.m_tiles, a.N, x3 ? 3 * a.K : a.K, sms, gran, gna ? 1 : (force_cluster == 1 || force_cluster == 2) ? force_cluster : 0,
-                                       (force_bn >= gran && force_bn <= 320 && force_bn % gran == 0 && a.N % force_bn == 0) ? force_bn : 0, allow_wide);
+                          choose_tiles(p.m_tiles, a.N, (planes == 3 ? 6 : planes == 2 ? 3 : 1) * a.K, sms, gran, gna ? 1 : (force_cluster == 1 || force_cluster == 2) ? force_cluster : 0,
+                                       (force_bn >= gran && force_bn <= (planes == 3 ? TC_X6_MAX_BN : 320) && force_bn % gran == 0 && a.N % force_bn == 0) ? force_bn : 0,
+                                       allow_wide, planes == 3 ? TC_X6_MAX_BN : 256);
     if (plan.block_n == 0) return fail(NMM_ERR_UNSUPPORTED, "tcgen05 GEMM: no N tile for N=%d", a.N);
     p.block_n = plan.block_n;
     p.cluster = plan.cluster;
@@ -1093,7 +1198,9 @@ int launch_linear_tc(const LinearArgs &a, cudaStream_t st) {
     p.n_tiles = a.N / p.block_n;
     p.cluster_tiles = m_groups * p.n_tiles;
     const size_t stage_bytes = (size_t)TC_A_BYTES + (size_t)(p.block_n / p.cluster) * TC_BK * 2;     // per CTA
-    p.epi_buf = (a.epilogue == NMM_EPI_RESIDUAL && a.out != nullptr && !a.no_h_store) ? 12288 : TC_EPI_BUF;
+    // a third 4 KB box: RESIDUAL writing h and a bf16 copy; PL 3 writing a third plane (GEGLU, RESIDUAL with `out`)
+    p.epi_buf = ((a.epilogue == NMM_EPI_RESIDUAL && a.out != nullptr && !a.no_h_store) ||
+                 (planes == 3 && a.out != nullptr && (a.epilogue == NMM_EPI_GEGLU || a.epilogue == NMM_EPI_RESIDUAL))) ? 12288 : TC_EPI_BUF;
     const size_t gn_coef = a.gn_x != nullptr ? (size_t)ceil_div(a.K, TC_BK) * TC_BK * 8 : 0;      // GNA: gamma | beta in shared memory
     const size_t fixed = 1024 /*alignment slack*/ + TC_BAR_BYTES + (size_t)TC_EPI_WARPS * p.epi_buf + gn_coef;
     int stages = (int)((TC_SMEM_MAX - fixed) / stage_bytes);
@@ -1105,7 +1212,7 @@ int launch_linear_tc(const LinearArgs &a, cudaStream_t st) {
     p.tmem_cols = cols;
     const size_t smem = fixed + (size_t)stages * stage_bytes;
     CUtensorMap ta, tw, th, to;
-    const int64_t kcols = x3 ? 2 * (int64_t)a.K : a.K;          // X3: [hi | lo] planes side by side
+    const int64_t kcols = planes * (int64_t)a.K;                 // PL > 1: [hi | lo] / [hi | mid | lo] planes side by side
     int rc = attn ? make_tmap_tokens_pf(&ta, a.A, a.attn_B, a.K, a.F, a.P, TC_BM / a.F)
              : gna ? make_tmap_x(&ta, a.gn_x, a.gn_B, a.K, a.F, a.P, a.xsb, a.xsc, a.xsf)
                  : make_tmap(&ta, a.A, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, a.M, kcols, kcols, TC_BM, TC_BK, CU_TENSOR_MAP_SWIZZLE_128B);
@@ -1120,7 +1227,7 @@ int launch_linear_tc(const LinearArgs &a, cudaStream_t st) {
         if (rc != NMM_OK) return rc;
     }
     if (a.out != nullptr && a.epilogue != NMM_EPI_OUTPUT && !attn) {
-        const int64_t ncols = (a.epilogue == NMM_EPI_GEGLU ? a.N / 2 : a.N) * (x3 ? 2 : 1);
+        const int64_t ncols = (a.epilogue == NMM_EPI_GEGLU ? a.N / 2 : a.N) * planes;
         rc = make_tmap(&to, a.out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, a.M, ncols, ncols, 32, 32, CU_TENSOR_MAP_SWIZZLE_64B);
         if (rc != NMM_OK) return rc;
     }
@@ -1144,9 +1251,12 @@ int launch_linear_tc(const LinearArgs &a, cudaStream_t st) {
         return launch_tc_t<NMM_EPI_STORE, 1, false, true>(ta, tw, th, to, p, e, smem, grid, st, fl, by, gn);
     }
 #define TC_DISPATCH(EPI)                                                                                   \
+    if (planes == 3)                                                                                       \
+        return p.cluster == 2 ? launch_tc_t<EPI, 2, false, false, 3>(ta, tw, th, to, p, e, smem, grid, st, fl, by)       \
+                              : launch_tc_t<EPI, 1, false, false, 3>(ta, tw, th, to, p, e, smem, grid, st, fl, by);      \
     if (x3)                                                                                                \
-        return p.cluster == 2 ? launch_tc_t<EPI, 2, false, false, true>(ta, tw, th, to, p, e, smem, grid, st, fl, by)    \
-                              : launch_tc_t<EPI, 1, false, false, true>(ta, tw, th, to, p, e, smem, grid, st, fl, by);   \
+        return p.cluster == 2 ? launch_tc_t<EPI, 2, false, false, 2>(ta, tw, th, to, p, e, smem, grid, st, fl, by)       \
+                              : launch_tc_t<EPI, 1, false, false, 2>(ta, tw, th, to, p, e, smem, grid, st, fl, by);      \
     if (lnf)                                                                                               \
         return p.cluster == 2 ? launch_tc_t<EPI, 2, true>(ta, tw, th, to, p, e, smem, grid, st, fl, by)    \
                               : launch_tc_t<EPI, 1, true>(ta, tw, th, to, p, e, smem, grid, st, fl, by);   \

@@ -187,8 +187,8 @@ int launch_gn_finalize(const Geo &g, const nmm_shape *s, const double *partial, 
 //   tokens[(bf*P + p), c] = (x[b,c,f,p] - mean[bf,g]) * rstd[bf,g] * gamma[c] + beta[c]
 // Generic kernel: 32(c) x 32(p) tile through shared memory, any dtype / alignment / ragged edges.
 // ------------------------------------------------------------------------------------------------
-// SPLIT (NMM_F32X3): tokens is a bf16 [N, 2C] tensor, every row = hi plane | lo plane of the fp32 values.
-template <typename T, bool SPLIT = false>
+// SPLIT = 2 (NMM_F32X3) / 3 (NMM_F32X6): tokens is a bf16 [N, SPLIT * C] tensor, every row = hi | lo (| mid | lo) planes of the fp32 values.
+template <typename T, int SPLIT = 0>
 __global__ void __launch_bounds__(256) gn_tokens_generic_kernel(const T *__restrict__ x, const double *__restrict__ partial,
                                                                 const float *__restrict__ gamma, const float *__restrict__ beta,
                                                                 T *__restrict__ tokens, int C, int F, int P, int splits, double count,
@@ -222,7 +222,7 @@ __global__ void __launch_bounds__(256) gn_tokens_generic_kernel(const T *__restr
     for (int i = 0; i < 4; i++) {
         int pl = ty + i * 8, p = p0 + pl, c = c0 + tx;
         if (c < C && p < P) {
-            if constexpr (SPLIT) split1_store(reinterpret_cast<bf16 *>(tokens) + ((int64_t)bf * P + p) * (2 * C), C, c, tile[tx][pl]);
+            if constexpr (SPLIT > 1) split1_store<SPLIT>(reinterpret_cast<bf16 *>(tokens) + ((int64_t)bf * P + p) * (SPLIT * C), C, c, tile[tx][pl]);
             else tokens[((int64_t)bf * P + p) * C + c] = from_f32<T>(tile[tx][pl]);
         }
     }
@@ -365,7 +365,10 @@ int launch_gn_tokens(const Geo &g, const nmm_shape *s, const Geo &full, const vo
         launch_pdl(gn_tokens_generic_kernel<bf16>, grid, 256, 0, st, (const bf16 *)x, partial, gn_w, gn_b, (bf16 *)tokens, g.C, g.F,
                    g.P, splits, count, s->eps_gn, s->x_stride_b, s->x_stride_c, s->x_stride_f);
     else if (g.dtype == NMM_F32X3)
-        launch_pdl(gn_tokens_generic_kernel<float, true>, grid, 256, 0, st, (const float *)x, partial, gn_w, gn_b, (float *)tokens, g.C, g.F,
+        launch_pdl(gn_tokens_generic_kernel<float, 2>, grid, 256, 0, st, (const float *)x, partial, gn_w, gn_b, (float *)tokens, g.C, g.F,
+                   g.P, splits, count, s->eps_gn, s->x_stride_b, s->x_stride_c, s->x_stride_f);
+    else if (g.dtype == NMM_F32X6)
+        launch_pdl(gn_tokens_generic_kernel<float, 3>, grid, 256, 0, st, (const float *)x, partial, gn_w, gn_b, (float *)tokens, g.C, g.F,
                    g.P, splits, count, s->eps_gn, s->x_stride_b, s->x_stride_c, s->x_stride_f);
     else
         launch_pdl(gn_tokens_generic_kernel<float>, grid, 256, 0, st, (const float *)x, partial, gn_w, gn_b, (float *)tokens, g.C, g.F,
@@ -467,6 +470,8 @@ __device__ __forceinline__ float half_warp_sum(float v) {
 }
 
 struct SplitOut { uint32_t pair; };      // tag (4 bytes per element like fp32): `out` is bf16 [N, 2C], row = hi plane | lo plane (NMM_F32X3)
+struct Split3Out { uint16_t t[3]; };     // tag (6 bytes per element): `out` is bf16 [N, 3C], row = hi | mid | lo planes (NMM_F32X6)
+template <typename TOut> constexpr int split_planes_of() { return std::is_same<TOut, SplitOut>::value ? 2 : std::is_same<TOut, Split3Out>::value ? 3 : 0; }
 
 template <typename TOut, int IT4>
 __global__ void __launch_bounds__(256) layernorm_pe_vec_kernel(const float *__restrict__ h, const float *__restrict__ gamma,
@@ -496,7 +501,7 @@ __global__ void __launch_bounds__(256) layernorm_pe_vec_kernel(const float *__re
     }
     const float rstd = rsqrtf(half_warp_sum(ss) * (1.0f / C) + eps);
     const float4 *per = pe ? reinterpret_cast<const float4 *>(pe + (int64_t)((row / P) % F) * C) : nullptr;
-    TOut *orow = out + row * C;               // (SplitOut: 4 bytes per element as well, so this is the row's hi plane)
+    TOut *orow = out + row * C;               // (SplitOut / Split3Out: 4 / 6 bytes per element, so this is the row's hi plane)
 #pragma unroll
     for (int i = 0; i < IT4; i++) {
         const int c4 = l16 + 16 * i;
@@ -507,7 +512,7 @@ __global__ void __launch_bounds__(256) layernorm_pe_vec_kernel(const float *__re
         o.z = fmaf((v[i].z - mu) * rstd, gm.z, bt.z); o.w = fmaf((v[i].w - mu) * rstd, gm.w, bt.w);
         if (per) { const float4 pp = __ldg(per + c4); o.x += pp.x; o.y += pp.y; o.z += pp.z; o.w += pp.w; }
         if (valid) {
-            if constexpr (std::is_same<TOut, SplitOut>::value) split4_store(reinterpret_cast<bf16 *>(orow), C, 4 * c4, o.x, o.y, o.z, o.w);
+            if constexpr (split_planes_of<TOut>() > 1) split4_store<split_planes_of<TOut>()>(reinterpret_cast<bf16 *>(orow), C, 4 * c4, o.x, o.y, o.z, o.w);
             else if constexpr (sizeof(TOut) == 2) reinterpret_cast<uint2 *>(orow)[c4] = make_uint2(pack_bf16x2(o.x, o.y), pack_bf16x2(o.z, o.w));
             else reinterpret_cast<float4 *>(orow)[c4] = o;
         }
@@ -536,7 +541,7 @@ __global__ void __launch_bounds__(256) layernorm_pe_generic_kernel(const float *
     for (int c = lane; c < C; c += 32) {
         float a = fmaf((hr[c] - mu) * rstd, gamma[c], beta[c]);
         if (per) a += per[c];
-        if constexpr (std::is_same<TOut, SplitOut>::value) split1_store(reinterpret_cast<bf16 *>(orow), C, c, a);
+        if constexpr (split_planes_of<TOut>() > 1) split1_store<split_planes_of<TOut>()>(reinterpret_cast<bf16 *>(orow), C, c, a);
         else orow[c] = from_f32<TOut>(a);
     }
 }
@@ -570,6 +575,7 @@ int launch_layernorm_pe(const Geo &g, const nmm_shape *s, const float *h, const 
                         void *out, cudaStream_t st) {
     if (g.dtype == NMM_BF16) return launch_ln_t<bf16>(g, s, h, w, b, pe, (bf16 *)out, st);
     if (g.dtype == NMM_F32X3) return launch_ln_t<SplitOut>(g, s, h, w, b, pe, (SplitOut *)out, st);
+    if (g.dtype == NMM_F32X6) return launch_ln_t<Split3Out>(g, s, h, w, b, pe, (Split3Out *)out, st);
     return launch_ln_t<float>(g, s, h, w, b, pe, (float *)out, st);
 }
 

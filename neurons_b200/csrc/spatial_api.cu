@@ -39,7 +39,7 @@ SpLayout sp_layout(const Geo &g, int ctx_dim) {
     SpLayout L;
     memset(&L, 0, sizeof(L));
     size_t off = 0;
-    const size_t C = g.C, D = ctx_dim, ws = g.dtype == NMM_F32X3 ? 4 : dtype_size(g.dtype);      // X3: bf16 [rows, 2 * cols]
+    const size_t C = g.C, D = ctx_dim, ws = operand_size(g.dtype);      // X3 / X6: bf16 [rows, 2 / 3 * cols]
     auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
     L.header = take(sizeof(SpHeader));
     L.gn_w = take(C * 4); L.gn_b = take(C * 4);
@@ -64,7 +64,7 @@ SpWork sp_work(const Geo &g, int ctx_len, int ctx_dim) {
     SpWork w;
     size_t off = 0;
     const size_t es = dtype_size(g.dtype);
-    const size_t opnd = g.dtype == NMM_F32X3 ? 4 : es;      // GEMM-operand element bytes (X3: two bf16 planes)
+    const size_t opnd = operand_size(g.dtype);      // GEMM-operand element bytes (X3 / X6: two / three bf16 planes)
     auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 1024); return o; };
     const size_t N = (size_t)g.N, C = g.C;
     w.gn_partial = take(gn_partial_bytes(g));
@@ -74,12 +74,13 @@ SpWork sp_work(const Geo &g, int ctx_len, int ctx_dim) {
     w.ctx = take(N * C * std::max(opnd, es));
     w.kv = take((size_t)g.B * ctx_len * 2 * C * 4);
     w.stat_part = take((N + 31) / 32 * C * sizeof(float2));      // N1: (sum, sum of squares) partials of y per 32-row block and channel
-    // NMM_F32X3: the fp32 attention output before it is split into hi | lo planes; the text states as hi | lo planes
-    w.ctx32 = take(g.dtype == NMM_F32X3 ? N * C * 4 : 0);
-    w.ehs2 = take(g.dtype == NMM_F32X3 ? (size_t)g.B * ctx_len * ctx_dim * 4 : 0);
-    // ... and q | k | v (self-attention) / q (cross-attention) and the text k | v as hi | lo planes for the fp32-grade attention kernel
-    w.qkv2 = take(g.dtype == NMM_F32X3 ? N * 3 * C * 4 : 0);
-    w.kv2 = take(g.dtype == NMM_F32X3 ? (size_t)g.B * ctx_len * 2 * C * 4 : 0);
+    // NMM_F32X3 / X6: the fp32 attention output before it is split into planes; the text states as planes
+    const bool split = planes_of(g.dtype) > 1;
+    w.ctx32 = take(split ? N * C * 4 : 0);
+    w.ehs2 = take(split ? (size_t)g.B * ctx_len * ctx_dim * opnd : 0);
+    // ... and q | k | v (self-attention) / q (cross-attention) and the text k | v as planes for the fp32-grade / fp32-exact attention kernel
+    w.qkv2 = take(split ? N * 3 * C * opnd : 0);
+    w.kv2 = take(split ? (size_t)g.B * ctx_len * 2 * C * opnd : 0);
     w.total = off;
     return w;
 }
@@ -91,6 +92,7 @@ int sp_validate(const nmm_spatial_shape *s) {
     int rc = nmm_validate(&b);
     if (rc != NMM_OK) return rc;
     if (b.dtype == NMM_F32X3 && s->ctx_dim % 64 != 0) return fail(NMM_ERR_UNSUPPORTED, "NMM_F32X3 needs ctx_dim %% 64 == 0 (got %d); use NMM_F32", s->ctx_dim);
+    if (b.dtype == NMM_F32X6 && s->ctx_dim % 64 != 0) return fail(NMM_ERR_UNSUPPORTED, "NMM_F32X6 needs ctx_dim %% 64 == 0 (got %d); use NMM_F32", s->ctx_dim);
     if (s->ctx_len <= 0 || s->ctx_dim <= 0 || s->ctx_dim % 8 != 0) return fail(NMM_ERR_BAD_ARG, "ctx_len / ctx_dim must be positive, ctx_dim %% 8 == 0");
     const int dh = b.channels / b.heads;
     if (dh != 40 && dh != 80 && dh != 160) return fail(NMM_ERR_UNSUPPORTED, "spatial transformer: head dim %d (supported: 40, 80, 160)", dh);
@@ -154,7 +156,7 @@ int nmm_spatial_pack_params(const nmm_spatial_shape *s, const nmm_spatial_params
         launch_pdl(sp_write_header_kernel, 1, 32, 0, st, hd, (SpHeader *)(base + L.header));
         NMM_LAUNCHED("sp_write_header_kernel");
     }
-    const size_t wsz = wd == NMM_F32X3 ? 4 : dtype_size(wd);      // X3: a row is its hi plane | lo plane (2 x bf16 per element)
+    const size_t wsz = operand_size(wd);      // X3 / X6: a row is its hi | lo (| mid | lo) planes (2 / 3 x bf16 per element)
     PACK(src->gn_w, L.gn_w, NMM_F32, C, 1, 0); PACK(src->gn_b, L.gn_b, NMM_F32, C, 1, 0);
     PACK(src->proj_in_w, L.w_in, wd, C, C, 0); PACK(src->proj_in_b, L.b_in, NMM_F32, C, 1, 0);      // Conv2d [C, C, 1, 1] == Linear [C, C]
     for (int l = 0; l < g.layers; l++) {
@@ -194,6 +196,11 @@ int nmm_spatial_attention(int32_t dtype, const void *q, const void *k, const voi
         if (q_row_stride % 2 || kv_row_stride % 2) return fail(NMM_ERR_BAD_ARG, "NMM_F32X3 spatial attention: row strides must be even (hi | lo planes)");
         a.q_lo_off = q_row_stride / 2; a.kv_lo_off = kv_row_stride / 2;
         return launch_spatial_attention_x3(a, (cudaStream_t)stream);
+    }
+    if (dtype == NMM_F32X6) {      // q, k, v: bf16 hi | mid | lo planes, each a third of a row stride after the previous one; o: fp32
+        if (q_row_stride % 3 || kv_row_stride % 3) return fail(NMM_ERR_BAD_ARG, "NMM_F32X6 spatial attention: row strides must be multiples of 3 (hi | mid | lo planes)");
+        a.q_lo_off = q_row_stride / 3; a.kv_lo_off = kv_row_stride / 3;
+        return launch_spatial_attention_x6(a, (cudaStream_t)stream);
     }
     return launch_spatial_attention(a, (cudaStream_t)stream);
 }
@@ -245,13 +252,15 @@ static int spatial_forward_impl(const nmm_spatial_shape *s, const void *x, const
     if ((rc = linear_dispatch(g.dtype, a, st)) != NMM_OK) return rc;
     a.gn_x = nullptr;
 
-    // NMM_F32X3 (fp32 activations, every Linear on the tensor cores as 3 bf16 MMAs): GEMM operands are hi | lo bf16 planes; q, k, v come out of
-    // their GEMMs as plain fp32 (STORE -> h-type buffer), the fp32 attention kernel's output is split into planes for to_out
-    const bool x3 = g.dtype == NMM_F32X3;
+    // NMM_F32X3 / X6 (fp32 activations, every Linear on the tensor cores as 3 / 6 bf16 MMAs): GEMM operands are hi | lo (| mid | lo) bf16 planes;
+    // q, k, v come out of their GEMMs as plain fp32 (STORE -> h-type buffer), the attention kernel's fp32 output is split into planes for to_out
+    const int pl = planes_of(g.dtype);
+    const bool x3 = pl > 1;
+    auto split_attention = [&](const FlashArgs &f) { return pl == 3 ? launch_spatial_attention_x6(f, st) : launch_spatial_attention_x3(f, st); };
     float *ctx32 = (float *)(ws + w.ctx32);
     const void *ehs_op = encoder_hidden_states;
     if (x3) {
-        if ((rc = launch_convert_rows(encoder_hidden_states, NMM_F32, ws + w.ehs2, NMM_F32X3, (int64_t)g.B * Lc, D, 0, st)) != NMM_OK) return rc;
+        if ((rc = launch_convert_rows(encoder_hidden_states, NMM_F32, ws + w.ehs2, g.dtype, (int64_t)g.B * Lc, D, 0, st)) != NMM_OK) return rc;
         ehs_op = ws + w.ehs2;
     }
     FlashArgs fa;
@@ -269,14 +278,14 @@ static int spatial_forward_impl(const nmm_spatial_shape *s, const void *x, const
         fa.q = big; fa.k = (const char *)big + (size_t)C * es; fa.v = (const char *)big + 2 * (size_t)C * es; fa.o = x3 ? (void *)ctx32 : ctx;
         fa.q_rs = fa.kv_rs = 3 * C; fa.o_rs = C; fa.q_bs = fa.kv_bs = (int64_t)P * 3 * C; fa.o_bs = (int64_t)P * C;
         fa.Lkv = P; fa.kv_div = 1;
-        if (x3) {          // q | k | v fp32 [N, 3C] -> planes [N, 6C] (hi: q | k | v, lo: q | k | v), fp32-grade attention on the tensor cores
+        if (x3) {          // q | k | v fp32 [N, 3C] -> planes [N, 3C * pl] (hi: q | k | v, (mid: q | k | v,) lo: q | k | v), attention on the tensor cores
             bf16 *qkv2 = (bf16 *)(ws + w.qkv2);
-            if ((rc = launch_convert_rows(big, NMM_F32, qkv2, NMM_F32X3, N, 3 * C, 0, st)) != NMM_OK) return rc;
+            if ((rc = launch_convert_rows(big, NMM_F32, qkv2, g.dtype, N, 3 * C, 0, st)) != NMM_OK) return rc;
             fa.q = qkv2; fa.k = qkv2 + C; fa.v = qkv2 + 2 * C;
-            fa.q_rs = fa.kv_rs = 6 * C; fa.q_bs = fa.kv_bs = (int64_t)P * 6 * C; fa.q_lo_off = fa.kv_lo_off = 3 * C;
-            if ((rc = launch_spatial_attention_x3(fa, st)) != NMM_OK) return rc;
+            fa.q_rs = fa.kv_rs = 3 * C * pl; fa.q_bs = fa.kv_bs = (int64_t)P * 3 * C * pl; fa.q_lo_off = fa.kv_lo_off = 3 * C;
+            if ((rc = split_attention(fa)) != NMM_OK) return rc;
         } else if ((rc = launch_spatial_attention(fa, st)) != NMM_OK) return rc;
-        if (x3 && (rc = launch_convert_rows(ctx32, NMM_F32, ctx, NMM_F32X3, N, C, 0, st)) != NMM_OK) return rc;
+        if (x3 && (rc = launch_convert_rows(ctx32, NMM_F32, ctx, g.dtype, N, C, 0, st)) != NMM_OK) return rc;
         a.epilogue = NMM_EPI_RESIDUAL; a.N = C; a.K = C; a.A = ctx; a.W = pk + o.wo1; a.bias = F32(o.bo1); a.h = h; a.out = nullptr;
         if ((rc = linear_dispatch(g.dtype, a, st)) != NMM_OK) return rc;
 
@@ -294,14 +303,14 @@ static int spatial_forward_impl(const nmm_spatial_shape *s, const void *x, const
         fa.Lkv = Lc; fa.kv_div = g.F;
         if (x3) {
             bf16 *q2 = (bf16 *)(ws + w.qkv2), *kv2 = (bf16 *)(ws + w.kv2);
-            if ((rc = launch_convert_rows(big, NMM_F32, q2, NMM_F32X3, N, C, 0, st)) != NMM_OK) return rc;
-            if ((rc = launch_convert_rows(kv, NMM_F32, kv2, NMM_F32X3, (int64_t)g.B * Lc, 2 * C, 0, st)) != NMM_OK) return rc;
+            if ((rc = launch_convert_rows(big, NMM_F32, q2, g.dtype, N, C, 0, st)) != NMM_OK) return rc;
+            if ((rc = launch_convert_rows(kv, NMM_F32, kv2, g.dtype, (int64_t)g.B * Lc, 2 * C, 0, st)) != NMM_OK) return rc;
             fa.q = q2; fa.k = kv2; fa.v = kv2 + C;
-            fa.q_rs = 2 * C; fa.q_bs = (int64_t)P * 2 * C; fa.q_lo_off = C;
-            fa.kv_rs = 4 * C; fa.kv_bs = (int64_t)Lc * 4 * C; fa.kv_lo_off = 2 * C;
-            if ((rc = launch_spatial_attention_x3(fa, st)) != NMM_OK) return rc;
+            fa.q_rs = C * pl; fa.q_bs = (int64_t)P * C * pl; fa.q_lo_off = C;
+            fa.kv_rs = 2 * C * pl; fa.kv_bs = (int64_t)Lc * 2 * C * pl; fa.kv_lo_off = 2 * C;
+            if ((rc = split_attention(fa)) != NMM_OK) return rc;
         } else if ((rc = launch_spatial_attention(fa, st)) != NMM_OK) return rc;
-        if (x3 && (rc = launch_convert_rows(ctx32, NMM_F32, ctx, NMM_F32X3, N, C, 0, st)) != NMM_OK) return rc;
+        if (x3 && (rc = launch_convert_rows(ctx32, NMM_F32, ctx, g.dtype, N, C, 0, st)) != NMM_OK) return rc;
         a.epilogue = NMM_EPI_RESIDUAL; a.N = C; a.K = C; a.A = ctx; a.W = pk + o.wo2; a.bias = F32(o.bo2); a.h = h; a.out = nullptr;
         if ((rc = linear_dispatch(g.dtype, a, st)) != NMM_OK) return rc;
 

@@ -14,7 +14,7 @@ LIB_PATH = os.path.join(HERE, os.environ.get("NMM_LIB", "libneurons_mm.so"))    
 NMM_MAX_LAYERS = 4
 NMM_MAX_ATTN = 4
 NMM_MAX_FRAMES = 32
-NMM_F32, NMM_BF16, NMM_F32X3 = 0, 1, 2
+NMM_F32, NMM_BF16, NMM_F32X3, NMM_F32X6 = 0, 1, 2, 3
 EPI_STORE, EPI_RESIDUAL, EPI_GEGLU, EPI_OUTPUT = 0, 1, 2, 3
 STATUS_NAMES = {0: "NMM_OK", -1: "NMM_ERR_BAD_ARG", -2: "NMM_ERR_UNSUPPORTED", -3: "NMM_ERR_WORKSPACE",
                 -4: "NMM_ERR_CUDA", -5: "NMM_ERR_DEVICE"}

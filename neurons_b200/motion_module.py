@@ -192,7 +192,8 @@ def config_of(module: nn.Module) -> ModuleConfig:
     return ModuleConfig(channels=channels, heads=int(a0.heads), layers=len(blocks), attn_blocks=len(b0.attention_blocks),
                         pos_enc=pos is not None, max_len=int(pos.pe.shape[1]) if pos is not None else 0,
                         ln_fold=bool(module.__dict__.get("_nmm_ln_fold", False)),      # set by tests / experiments before the first call
-                        fp32_tc=not bool(module.__dict__.get("_nmm_fp32_fma", False)))  # fp32 activations: tensor cores (3 x bf16) unless set
+                        fp32_tc=not bool(module.__dict__.get("_nmm_fp32_fma", False)),  # fp32 activations: tensor cores (3 x bf16) unless set
+                        fp32_exact=ops.fp32_exact_selected(module))                       # fp32 activations: 6 x bf16 (exact), raises with the FMA flag
 
 
 def _param_tensors(module: nn.Module) -> Dict[str, torch.Tensor]:
@@ -226,7 +227,8 @@ class _Engine:
     @staticmethod
     def _flags(module):
         # per-module mode switches that change the packed layout: part of the key, so flipping one re-packs instead of being ignored
-        return (bool(module.__dict__.get("_nmm_ln_fold", False)), bool(module.__dict__.get("_nmm_fp32_fma", False)))
+        return (bool(module.__dict__.get("_nmm_ln_fold", False)), bool(module.__dict__.get("_nmm_fp32_fma", False)),
+                bool(module.__dict__.get("_nmm_fp32_exact", False)))
 
     @staticmethod
     def _checksum(tensors):

@@ -36,13 +36,30 @@ class ModuleConfig:
     # fp32 activations: True = every Linear on the tensor cores as 3 bf16 MMAs per product (NMM_F32X3; needs channels % 64 == 0,
     # other widths use the FMA path); False (or env NMM_FP32_FMA=1) = the fp32 FMA-pipe GEMM (NMM_F32), kept as the checker.
     fp32_tc: bool = True
+    # fp32 activations, exact: 6 bf16 MMAs per product over three-plane splits (NMM_F32X6; channels % 64 == 0), as accurate as the FMA
+    # path; other widths use the FMA path, which is exact too.  Module flag `_nmm_fp32_exact` or env NMM_FP32_EXACT=1.
+    fp32_exact: bool = False
 
 
 _FP32_FMA_ENV = os.environ.get("NMM_FP32_FMA")     # read ONCE at import (pack and forward must agree on the mode)
+_FP32_EXACT_ENV = os.environ.get("NMM_FP32_EXACT")
+
+
+def fp32_exact_selected(module) -> bool:
+    """Is the fp32-exact mode selected for this module (flag `_nmm_fp32_exact` or env NMM_FP32_EXACT=1)?  Raises when the FMA mode is
+    selected for it too (flag `_nmm_fp32_fma` or env NMM_FP32_FMA=1): both are exact, and the choice between them is not made silently."""
+    exact = bool(module.__dict__.get("_nmm_fp32_exact", False)) or _FP32_EXACT_ENV not in (None, "0")
+    fma = bool(module.__dict__.get("_nmm_fp32_fma", False)) or _FP32_FMA_ENV not in (None, "0")
+    if exact and fma:
+        raise ValueError("neurons_b200: both the fp32-exact tensor-core mode (_nmm_fp32_exact / NMM_FP32_EXACT) and the FMA mode "
+                         "(_nmm_fp32_fma / NMM_FP32_FMA) are selected for this module; select one")
+    return exact
 
 
 def _dtype_code(dt: torch.dtype, cfg: Optional["ModuleConfig"] = None) -> int:
     if dt == torch.float32:
+        if cfg is not None and cfg.fp32_exact:
+            return _lib.NMM_F32X6 if cfg.channels % 64 == 0 else _lib.NMM_F32
         if cfg is not None and cfg.fp32_tc and cfg.channels % 64 == 0 and _FP32_FMA_ENV in (None, "0"):
             return _lib.NMM_F32X3
         return _lib.NMM_F32
@@ -436,31 +453,46 @@ def temporal_attention(cfg: ModuleConfig, dims, qkv: torch.Tensor) -> torch.Tens
     return ctx
 
 
-def split_planes(t: torch.Tensor) -> torch.Tensor:
-    """fp32 [rows, K] -> the NMM_F32X3 operand format: bf16 [rows, 2K], row = hi plane | lo plane (t = hi + lo + O(2^-17 t))."""
-    hi = t.to(torch.bfloat16)
-    lo = (t.float() - hi.float()).to(torch.bfloat16)
-    return torch.cat([hi, lo], dim=1).contiguous()
+def split_planes(t: torch.Tensor, planes: int = 2) -> torch.Tensor:
+    """fp32 [rows, K] -> the NMM_F32X3 operand format (planes=2): bf16 [rows, 2K], row = hi plane | lo plane (t = hi + lo + O(2^-17 t)),
+    or the NMM_F32X6 format (planes=3): bf16 [rows, 3K], row = hi | mid | lo, hi = bf16(t), mid = bf16(t - hi), lo = bf16(t - hi - mid)
+    (each difference in fp32, where it is exact; t = hi + mid + lo + O(2^-24 t))."""
+    if planes not in (2, 3):
+        raise ValueError(f"split_planes: planes must be 2 or 3, got {planes}")
+    r = t.float()
+    out = []
+    for _ in range(planes):
+        p = r.to(torch.bfloat16)
+        out.append(p)
+        r = r - p.float()
+    return torch.cat(out, dim=1).contiguous()
 
 
-def merge_planes(t: torch.Tensor) -> torch.Tensor:
-    k = t.shape[1] // 2
-    return t[:, :k].float() + t[:, k:].float()
+def merge_planes(t: torch.Tensor, planes: int = 2) -> torch.Tensor:
+    k = t.shape[1] // planes
+    out = t[:, :k].float()
+    for i in range(1, planes):
+        out = out + t[:, i * k:(i + 1) * k].float()
+    return out
 
 
 def linear(A: torch.Tensor, Wt: torch.Tensor, bias: Optional[torch.Tensor] = None, epilogue: int = _lib.EPI_STORE,
            h: Optional[torch.Tensor] = None, want_out: bool = True, cfg: Optional[ModuleConfig] = None,
-           x: Optional[torch.Tensor] = None, x3: bool = False) -> Optional[torch.Tensor]:
+           x: Optional[torch.Tensor] = None, x3: bool = False, x6: bool = False) -> Optional[torch.Tensor]:
     """D = A . Wt^T with a fused epilogue (see include/neurons_mm.h nmm_epilogue).  A: [M,K], Wt: [N,K].
-    x3=True (fp32 A / Wt): the 3 x bf16 tensor-core mode -- operands are converted to hi | lo planes here, `out` is merged back to fp32."""
+    x3=True (fp32 A / Wt): the 3 x bf16 tensor-core mode -- operands are converted to hi | lo planes here, `out` is merged back to fp32.
+    x6=True (fp32 A / Wt): the 6 x bf16 (fp32-exact) tensor-core mode, the same with hi | mid | lo planes."""
     _require_cuda(A, "A")
     A, Wt = A.contiguous(), Wt.contiguous()
     M, K = A.shape
     N = Wt.shape[0]
     dt = _dtype_code(A.dtype)
-    if x3:
+    if x3 and x6:
+        raise ValueError("linear: x3 and x6 are exclusive")
+    planes = 3 if x6 else 2 if x3 else 1
+    if planes > 1:
         assert A.dtype == torch.float32 and Wt.dtype == torch.float32
-        A, Wt, dt = split_planes(A), split_planes(Wt), _lib.NMM_F32X3
+        A, Wt, dt = split_planes(A, planes), split_planes(Wt, planes), (_lib.NMM_F32X6 if x6 else _lib.NMM_F32X3)
     bias_ptr = None
     if bias is not None:
         bias = bias.float().contiguous()
@@ -479,12 +511,12 @@ def linear(A: torch.Tensor, Wt: torch.Tensor, bias: Optional[torch.Tensor] = Non
         out_ptr = None
     else:
         if want_out:
-            out = torch.empty((M, (N // 2 if epilogue == _lib.EPI_GEGLU else N) * (2 if x3 else 1)), dtype=A.dtype, device=A.device)
+            out = torch.empty((M, (N // 2 if epilogue == _lib.EPI_GEGLU else N) * planes), dtype=A.dtype, device=A.device)
         out_ptr = out.data_ptr() if out is not None else None
     h_ptr = h.data_ptr() if h is not None else None
     with torch.cuda.device(A.device):
         _lib.check(_lib.load().nmm_linear(dt, epilogue, M, N, K, A.data_ptr(), Wt.data_ptr(), bias_ptr, h_ptr, out_ptr, shape_ref,
                                           x_ptr, y_ptr, _stream_ptr(A.device)))
-    if x3 and out is not None and epilogue != _lib.EPI_OUTPUT:
-        out = merge_planes(out)
+    if planes > 1 and out is not None and epilogue != _lib.EPI_OUTPUT:
+        out = merge_planes(out, planes)
     return out

@@ -41,6 +41,9 @@ class SpatialConfig:
     # False (module flag `_nmm_fp32_fma` or env NMM_FP32_FMA=1) = the FMA-pipe GEMM (NMM_F32) and fp32 attention on the FMA pipe (no bf16
     # rounding anywhere; the tiled flash kernel at every UNet size, the one-warp-per-query checker kernel for small shapes).
     fp32_tc: bool = True
+    # fp32 activations, exact (module flag `_nmm_fp32_exact` or env NMM_FP32_EXACT=1): every Linear and the attention as 6 bf16 MMAs per
+    # product over three-plane splits (NMM_F32X6; channels, ctx_dim % 64 == 0, other widths use the FMA path, which is exact too)
+    fp32_exact: bool = False
 
 
 class Transformer3DModelOutput:
@@ -131,11 +134,13 @@ def spatial_config_of(module: nn.Module) -> SpatialConfig:
     if channels // heads not in (40, 80, 160):
         raise NotImplementedError(f"neurons_b200: spatial attention head dim {channels // heads} (supported: 40, 80, 160)")
     return SpatialConfig(channels=channels, heads=heads, layers=len(blocks), ctx_dim=int(b0.attn2.to_k.in_features),
-                         fp32_tc=not bool(module.__dict__.get("_nmm_fp32_fma", False)))
+                         fp32_tc=not bool(module.__dict__.get("_nmm_fp32_fma", False)), fp32_exact=ops.fp32_exact_selected(module))
 
 
 def _dtype_code(dt: torch.dtype, cfg: Optional["SpatialConfig"] = None) -> int:
     if dt == torch.float32:
+        if cfg is not None and cfg.fp32_exact:
+            return _lib.NMM_F32X6 if cfg.channels % 64 == 0 and cfg.ctx_dim % 64 == 0 else _lib.NMM_F32
         if cfg is not None and cfg.fp32_tc and cfg.channels % 64 == 0 and cfg.ctx_dim % 64 == 0 and ops._FP32_FMA_ENV in (None, "0"):
             return _lib.NMM_F32X3
         return _lib.NMM_F32
@@ -242,13 +247,15 @@ def spatial_forward_packed(x: torch.Tensor, encoder_hidden_states: torch.Tensor,
     return out
 
 
-def spatial_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int, kv_div: int = 1, x3: bool = False) -> torch.Tensor:
+def spatial_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: int, kv_div: int = 1, x3: bool = False,
+                      x6: bool = False) -> torch.Tensor:
     """Per-stage entry (tests / micro-benchmarks): q [images, Lq, heads*dh], k / v [images / kv_div, Lkv, heads*dh] (last dim dense; row
     and image strides free) -> o [images, Lq, heads*dh].  nmm_spatial_attention.
     fp32 q, k, v (x3=False): fp32 throughout on the FMA pipe, the attention of the FMA mode -- the tiled flash kernel from 2^17 score elements
     (Lq * Lkv * images * heads) up, the checker kernel below; q, k, v need 16-byte alignment and strides in multiples of 4 for the tiled kernel.
     x3=True (fp32 q, k, v): the fp32-grade tensor-core kernel of the NMM_F32X3 mode -- q and k | v are converted to hi | lo planes here
-    (like ops.linear(..., x3=True)); o is fp32."""
+    (like ops.linear(..., x3=True)); o is fp32.
+    x6=True (fp32 q, k, v): the fp32-exact tensor-core kernel of the NMM_F32X6 mode -- the same with hi | mid | lo planes."""
     for t, name in ((q, "q"), (k, "k"), (v, "v")):
         ops._require_cuda(t, name)
         if t.dim() != 3 or t.stride(2) != 1:
@@ -257,14 +264,17 @@ def spatial_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, heads: 
     if k.shape != v.shape or k.stride() != v.stride() or k.shape[0] * kv_div != images or k.shape[2] != Cc:
         raise ValueError("k / v must share shape and strides, with images == kv images * kv_div")
     dt = _dtype_code(q.dtype)
-    if x3:
+    if x3 and x6:
+        raise ValueError("spatial_attention: x3 and x6 are exclusive")
+    pl = 3 if x6 else 2 if x3 else 1
+    if pl > 1:
         if q.dtype != torch.float32 or k.dtype != torch.float32 or v.dtype != torch.float32:
-            raise TypeError("spatial_attention(x3=True) takes fp32 q, k, v")
+            raise TypeError(f"spatial_attention(x{2 * pl}=True) takes fp32 q, k, v")
         Lkv = k.shape[1]
-        q = ops.split_planes(q.reshape(images * Lq, Cc)).view(images, Lq, 2 * Cc)                      # rows [hi q | lo q]
-        kv = ops.split_planes(torch.cat([k, v], -1).reshape(-1, 2 * Cc)).view(-1, Lkv, 4 * Cc)        # rows [hi k | hi v | lo k | lo v]
-        k, v, dt = kv[..., :Cc], kv[..., Cc:2 * Cc], _lib.NMM_F32X3
-    o = torch.empty((images, Lq, Cc), dtype=torch.float32 if x3 else q.dtype, device=q.device)
+        q = ops.split_planes(q.reshape(images * Lq, Cc), pl).view(images, Lq, pl * Cc)                  # rows [hi q | (mid q |) lo q]
+        kv = ops.split_planes(torch.cat([k, v], -1).reshape(-1, 2 * Cc), pl).view(-1, Lkv, 2 * pl * Cc)  # rows [hi k | hi v | ... | lo k | lo v]
+        k, v, dt = kv[..., :Cc], kv[..., Cc:2 * Cc], (_lib.NMM_F32X6 if x6 else _lib.NMM_F32X3)
+    o = torch.empty((images, Lq, Cc), dtype=torch.float32 if pl > 1 else q.dtype, device=q.device)
     with torch.cuda.device(q.device):
         _lib.check(_lib.load().nmm_spatial_attention(dt, q.data_ptr(), k.data_ptr(), v.data_ptr(), o.data_ptr(), q.stride(1), k.stride(1),
                                                      o.stride(1), q.stride(0), k.stride(0), o.stride(0), Lq, k.shape[1], heads, Cc // heads, images,
