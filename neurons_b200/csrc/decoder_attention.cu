@@ -37,21 +37,25 @@ __global__ void __launch_bounds__(128) gn_time_tokens_kernel(const T *__restrict
     if (i >= (int64_t)B * NMM_GN_GROUPS * P) return;
     const int p = (int)(i % P), g = (int)((i / P) % NMM_GN_GROUPS), b = (int)(i / ((int64_t)P * NMM_GN_GROUPS));
     const T *xb = x + (int64_t)b * sb + p;
+    // The frames of a decoded video are close to each other, so a group (cpg channels x t frames at one position) often has a variance
+    // far below mean^2, where sq / n - mean^2 on raw values cancels away every significant bit.  Shifting by the group's first value K
+    // keeps the sums of v - K well conditioned, and the values are normalised as (v - K) - mean_d without rounding the mean K + mean_d.
+    const float K = to_f32(xb[(int64_t)(g * cpg) * sc]);
     float sum = 0.f, sq = 0.f;
     for (int f = 0; f < F; f++)
         for (int j = 0; j < cpg; j++) {
-            const float v = to_f32(xb[(int64_t)f * sf + (int64_t)(g * cpg + j) * sc]);
-            sum += v; sq += v * v;
+            const float d = to_f32(xb[(int64_t)f * sf + (int64_t)(g * cpg + j) * sc]) - K;
+            sum += d; sq = fmaf(d, d, sq);
         }
     const float n = (float)(F * cpg);
-    const float mean = sum / n;
-    const float var = fmaxf(sq / n - mean * mean, 0.f);
+    const float mean_d = sum / n;
+    const float var = fmaxf(sq / n - mean_d * mean_d, 0.f);
     const float rstd = rsqrtf(var + eps);
     for (int f = 0; f < F; f++)
         for (int j = 0; j < cpg; j++) {
             const int c = g * cpg + j;
-            const float v = to_f32(xb[(int64_t)f * sf + (int64_t)c * sc]);
-            tokens[((int64_t)(b * F + f) * P + p) * C + c] = from_f32<T>((v - mean) * rstd * gamma[c] + beta[c]);
+            const float d = to_f32(xb[(int64_t)f * sf + (int64_t)c * sc]) - K;
+            tokens[((int64_t)(b * F + f) * P + p) * C + c] = from_f32<T>((d - mean_d) * rstd * gamma[c] + beta[c]);
         }
 }
 

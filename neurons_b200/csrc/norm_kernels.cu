@@ -50,20 +50,29 @@ template <typename T> struct Vec16;   // 16-byte vector of T
 template <> struct Vec16<float> { static constexpr int N = 4; };
 template <> struct Vec16<bf16> { static constexpr int N = 8; };
 
+// Accumulation of the 16 bytes of one vector on the packed fp32x2 pipe: d = v - K, s += d, ss += d * d with two accumulator lanes
+// (even / odd elements of the vector), nK2 = (-K, -K) (K = 0 for bf16: d = v exactly).  Three packed instructions per element pair.
 template <typename T>
-__device__ __forceinline__ void accum16v(const uint4 v, float &s, float &ss) {
+__device__ __forceinline__ void accum16v(const uint4 v, uint64_t nK2, uint64_t &s2, uint64_t &ss2) {
     if constexpr (sizeof(T) == 4) {
-        float f[4] = {__uint_as_float(v.x), __uint_as_float(v.y), __uint_as_float(v.z), __uint_as_float(v.w)};
-#pragma unroll
-        for (int i = 0; i < 4; i++) { s += f[i]; ss = fmaf(f[i], f[i], ss); }
+        const uint64_t d0 = f32x2_add(f32x2_pack(__uint_as_float(v.x), __uint_as_float(v.y)), nK2);
+        const uint64_t d1 = f32x2_add(f32x2_pack(__uint_as_float(v.z), __uint_as_float(v.w)), nK2);
+        s2 = f32x2_add(s2, d0); ss2 = f32x2_fma(d0, d0, ss2);
+        s2 = f32x2_add(s2, d1); ss2 = f32x2_fma(d1, d1, ss2);
     } else {
-        uint32_t w[4] = {v.x, v.y, v.z, v.w};
+        const uint32_t w[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
         for (int i = 0; i < 4; i++) {
-            float a = bf16_lo(w[i]), b = bf16_hi(w[i]);
-            s += a + b; ss = fmaf(a, a, ss); ss = fmaf(b, b, ss);
+            const uint64_t d = f32x2_add(f32x2_pack(bf16_lo(w[i]), bf16_hi(w[i])), nK2);
+            s2 = f32x2_add(s2, d); ss2 = f32x2_fma(d, d, ss2);
         }
     }
+}
+
+__device__ __forceinline__ double warp_sum_d(double v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
 }
 
 // VEC: PT 16-byte vectors per thread (chunk = blockDim.x * PT vectors); !VEC: element loop over the same chunk.
@@ -84,8 +93,24 @@ __global__ void __launch_bounds__(GN_MAX_THREADS) gn_stats_kernel(const T *__res
     const int64_t chunk = (int64_t)blockDim.x * PT * 8;                 // elements per CTA (8 = bf16 per vector; the fp32 path covers it in 2 PT rounds)
     const int64_t e0 = (int64_t)split * chunk;
     const int64_t e1 = min(total, e0 + chunk);
+    // One-pass sums of x and x^2 lose (|mean| / std)^2 of relative accuracy in the variance once they are rounded, and the cancellation
+    // in c2 / count - mean^2 comes after.  So each thread's fp32 sums go to double before any sum over threads, and:
+    //  * fp32 input: every thread accumulates x - K, K = the fp32 mean of the first min(P, 8) elements of the group (the same value in
+    //    every thread and split), which keeps the per-thread sums well conditioned whatever the offset;
+    //  * bf16 input: no shift.  x^2 of a bf16 value has 16 significant bits, so a thread's fp32 sums of <= 128 of them are exact whenever
+    //    the values share an exponent range -- which an offset group does -- and a shift would only add rounding.
+    auto shift_of = [&]() {                            // broadcast loads (L1 / L2 after the first warp)
+        if constexpr (sizeof(T) != 4) return 0.f;
+        const int nk = P < 8 ? P : 8;
+        float acc = 0.f;
+        for (int j = 0; j < nk; j++) acc += to_f32(__ldg(base + j));
+        return acc / (float)nk;
+    };
+    float K = 0.f;
     float s = 0.f, ss = 0.f;
+    int n = 0;                                         // valid elements this thread accumulated
     if constexpr (VEC) {
+        uint64_t s2 = f32x2_pack(0.f, 0.f), ss2 = s2, nK2 = s2;
         const int tot = (int)total;                    // cpg*P < 2^31 (validated); P % V == 0, so a vector never straddles channels
         constexpr int ROUNDS = 8 / V;                   // fp32: 4 elements per vector -> two rounds of PT loads cover the same chunk
 #pragma unroll
@@ -93,6 +118,7 @@ __global__ void __launch_bounds__(GN_MAX_THREADS) gn_stats_kernel(const T *__res
             const int base_e = (int)e0 + rd * (int)blockDim.x * PT * V;
             // issue every load of this round before the first accumulate
             uint4 v[PT];
+            uint32_t ok_mask = 0;
 #pragma unroll
             for (int i = 0; i < PT; i++) {
                 const int e = base_e + (i * (int)blockDim.x + (int)threadIdx.x) * V;
@@ -100,20 +126,32 @@ __global__ void __launch_bounds__(GN_MAX_THREADS) gn_stats_kernel(const T *__res
                 const int c = ok ? e / P : 0;
                 const int p = ok ? e - c * P : 0;
                 v[i] = ok ? __ldg(reinterpret_cast<const uint4 *>(base + (int64_t)c * sc + p)) : make_uint4(0u, 0u, 0u, 0u);
+                ok_mask |= (uint32_t)ok << i;
+            }
+            if (rd == 0) {                              // once this round's loads are in flight
+                K = shift_of();
+                nK2 = f32x2_pack(-K, -K);
             }
 #pragma unroll
-            for (int i = 0; i < PT; i++) accum16v<T>(v[i], s, ss);      // zero vectors add nothing
+            for (int i = 0; i < PT; i++)
+                if (ok_mask >> i & 1u) { accum16v<T>(v[i], nK2, s2, ss2); n += V; }     // a lane past the group's end adds nothing, not (0 - K)^2
         }
+        float a0, a1;
+        f32x2_unpack(s2, a0, a1); s = a0 + a1;
+        f32x2_unpack(ss2, a0, a1); ss = a0 + a1;
     } else {
+        K = shift_of();
         for (int64_t e = e0 + threadIdx.x; e < e1; e += blockDim.x) {
             int c = (int)(e / P); int p = (int)(e - (int64_t)c * P);
-            float v = to_f32(base[(int64_t)c * sc + p]);
-            s += v; ss = fmaf(v, v, ss);
+            const float d = to_f32(base[(int64_t)c * sc + p]) - K;
+            s += d; ss = fmaf(d, d, ss); n++;
         }
     }
-    // block reduce in double (per-thread fp32 partials cover <= 128 elements each)
+    // un-shift per thread in double (s, ss, K are fp32 and n <= 128, so only double roundings remain), then reduce in double:
+    //   sum x = s + n K,  sum x^2 = ss + 2 K s + n K^2
     __shared__ double sh[2][GN_MAX_THREADS / 32];
-    double ds = (double)warp_sum(s), dss = (double)warp_sum(ss);
+    const double dK = (double)K, dsh = (double)s;
+    const double ds = warp_sum_d(fma((double)n, dK, dsh)), dss = warp_sum_d(fma((double)n * dK, dK, fma(2.0 * dK, dsh, (double)ss)));
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (lane == 0) { sh[0][warp] = ds; sh[1][warp] = dss; }
     __syncthreads();
@@ -278,11 +316,6 @@ __global__ void __launch_bounds__(256) gn_tokens_bf16_kernel(const bf16 *__restr
 // these kernels reduce them -- one warp per (b, f, group), fixed order, double accumulation, no atomics -- to the
 // [B*F*32][2] double "sums" format every GroupNorm consumer of the library accepts as precomputed statistics.
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ double warp_sum_d(double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
 // part[tile][F][32] (fused module kernel; tile = b * tiles_per_b + tt)
 __global__ void __launch_bounds__(256) y_sums_from_tiles_kernel(const float2 *__restrict__ part, double *__restrict__ sums, int F, int tiles_per_b, int n) {
     pdl_wait();

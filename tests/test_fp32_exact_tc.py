@@ -264,17 +264,24 @@ def test_x6_attention_vs_fp64(kw, Lq, Lkv, dh, kv_div):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", __import__("tests.helpers", fromlist=["golden_names"]).golden_names())
-def test_motion_module_golden_x6(name):
+def test_motion_module_golden_x6_vs_fp64(name):
+    """Both exact modes within the fp32 bar of the fixture's fp32 reference output, and x6 within 2x the FMA mode's error against the
+    oracle in fp64.  (Against the fp32 reference both errors are 1-2e-6, the size of that reference's own rounding: at c320_f8_8x8_a2 the
+    x6 mode's worst element is 2.4e-6 from the fp32 reference, which is itself 1.4e-6 from fp64 there.)"""
+    from oracle import motion_oracle as mo
     from tests import helpers
     fx, cfg, params, x = helpers.load_golden(name)
-    errs = {}
+    ref64 = mo.forward_reference_order({k: v.double() for k, v in params.items()}, x.double(), cfg)
+    errs, errs64 = {}, {}
     with torch.no_grad():
         for flag in ("_nmm_fp32_fma", "_nmm_fp32_exact"):
             m = helpers.mirror_module(cfg, params, "cuda")
             m.__dict__[flag] = True
-            errs[flag] = _maxabs(m(x.cuda(), None, None), fx["out_ref_fp32"])
-    print(name, errs)
-    assert errs["_nmm_fp32_exact"] <= TOL_FP32 and errs["_nmm_fp32_exact"] <= 2.0 * errs["_nmm_fp32_fma"], errs
+            y = m(x.cuda(), None, None)
+            errs[flag], errs64[flag] = _maxabs(y, fx["out_ref_fp32"]), _maxabs(y, ref64)
+    print(name, errs, errs64)
+    assert errs["_nmm_fp32_exact"] <= TOL_FP32 and errs["_nmm_fp32_fma"] <= TOL_FP32, errs
+    assert errs64["_nmm_fp32_exact"] <= 2.0 * errs64["_nmm_fp32_fma"], errs64
 
 
 def _sp_mirror(cfg, params, flag):
